@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py - env-steps/sec of the lockstep ReachBall step path (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N --steps K --warmup W
 
 A "step" is one launch of the fused step kernel over one batch of synthetic actions: 2^20 ReachBall episodes per
@@ -25,6 +25,11 @@ region.  One JSON line is printed by rank 0.
 --impl reference times that CPU oracle alone on the SAME workload (2^20 envs x 16 cycles per step).  The reference's own
 step path needs rcssserver + the C++ proxy, external binaries that cannot run offline; the oracle is the CPU restatement
 of the same path.  That arm imports neither the product package nor libsoccer2d.so.
+
+--dump-outputs DIR writes what the last timed launch of the B200 arm returned (rank 0's envs): obs.npy, reward.npy,
+done.npy, result.npy as float32, and env_index.npy (float64), the env of each row.  Actions and the env seed are fixed,
+so two builds run with the same arguments can be compared output for output.  Above 64 MB a fixed, seeded sample of
+the envs is written.
 """
 import argparse
 import json
@@ -47,6 +52,7 @@ SCENARIO_KW = dict(use_continuous_action=False, action_space_size=16, change_bal
                    change_ball_velocity=True, min_distance_to_ball=5.0, max_steps=200)
 STATE_BYTES, OBS_BYTES, OUT_BYTES = 80, 40, 6  # per env: state planes; obs row; reward + done + result
 FG_STATE_BYTES, FG_OBS_BYTES = 22 * 36 + 80, 480  # per 11v11 match: 22 players x 9 words + 16 match words + 16 B of tackle / catch counters
+DUMP_BYTES = 64 * 10**6 - 4096  # --dump-outputs budget, less room for the .npy headers
 
 
 def algorithmic_bytes_per_env(k):
@@ -214,6 +220,21 @@ def time_launches(env, pool, steps, flush):
     return [s.elapsed_time(e) for s, e in zip(starts, stops)]
 
 
+def dump_outputs(out_dir, obs, reward, done, result):
+    """the step's (obs, reward, done, result) as float32 .npy files under out_dir, with the env index of every row;
+    a seeded sample of the envs (the same rows in every file) when all of them would exceed DUMP_BYTES"""
+    import numpy as np
+    n = reward.shape[0]
+    per_env = 4 * (obs[0].numel() + 3) + 8
+    rows = np.arange(n)
+    if n * per_env > DUMP_BYTES:
+        rows = np.sort(np.random.default_rng(0).choice(n, DUMP_BYTES // per_env, replace=False))
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in (("obs", obs), ("reward", reward), ("done", done), ("result", result)):
+        np.save(os.path.join(out_dir, f"{name}.npy"), t.cpu().numpy()[rows].astype(np.float32))
+    np.save(os.path.join(out_dir, "env_index.npy"), rows.astype(np.float64))
+
+
 class Ranks:
     """barrier / max-over-ranks of the timing contract"""
 
@@ -326,10 +347,10 @@ def commands(torch, gen, dev, shape):
     return a
 
 
-def measure_scenario(kind, total, k, steps, warmup, rank, world, dev, ranks, numa_node, with_e2e=True):
+def measure_scenario(kind, total, k, steps, warmup, rank, world, dev, ranks, numa_node, with_e2e=True, dump_dir=None):
     """BASELINE configs[2] (kind = "shoot": 1v0 shoot-on-goal, `total` envs) / configs[3] ("fullgame": 11v11, `total`
     matches), sharded over the ranks (strong scaling, shard_range), command actions resident in HBM.  Same timing rules
-    as the main arm.  Returns the section dict (identical on every rank)."""
+    as the main arm; `dump_dir`: see dump_outputs.  Returns the section dict (identical on every rank)."""
     import torch
 
     from soccer2d_b200 import Soccer2DVecEnv, shard_range
@@ -361,6 +382,8 @@ def measure_scenario(kind, total, k, steps, warmup, rank, world, dev, ranks, num
     ranks.barrier()
     total_ms = ranks.max(sum(ms))
     launch_ms = sum(ms) / len(ms)
+    if dump_dir:
+        dump_outputs(dump_dir, env.obs, env.reward, env.done, env.result)
     out = {"workload": name, "value": total * k * steps / (total_ms * 1e-3), "unit": UNIT, "scaling": "strong",
            "envs_per_gpu": n, "global_envs": total, "substeps": k, "steps": steps, "launch_ms": launch_ms,
            "ms_per_step": total_ms / steps, "gpu_launches": steps}
@@ -422,7 +445,8 @@ def run_b200(args, rank, local_rank, world):
         total = args.envs if args.envs != ENVS_PER_GPU else (1 << 22 if args.workload == "shoot" else 1 << 18)
         sampler = ClockSampler(local_rank)
         sampler.start()
-        sec = measure_scenario(args.workload, total, args.substeps, args.steps, args.warmup, rank, world, dev, ranks, numa_node)
+        sec = measure_scenario(args.workload, total, args.substeps, args.steps, args.warmup, rank, world, dev, ranks, numa_node,
+                               dump_dir=args.dump_outputs if rank == 0 else None)
         clocks = sampler.summary()
         if rank == 0:
             line = {"metric": METRIC, "value": sec["value"], "unit": UNIT, "n_gpus": world, "steps": args.steps,
@@ -456,6 +480,8 @@ def run_b200(args, rank, local_rank, world):
     total_ms = ranks.max(sum(ms))
     value = world * n * k * args.steps / (total_ms * 1e-3)
     launch_ms = sum(ms) / len(ms)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, env.obs, env.reward, env.done, env.result)  # what the last step_torch returned
 
     # ---- e2e: host buffers, every step's actions H2D and results D2H inside the timed region --------------
     host_pool = [env.pinned_like(p) for p in pool[:3]]
@@ -632,7 +658,7 @@ def run_b200(args, rank, local_rank, world):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=200)
+    ap.add_argument("--steps", type=int, default=None, help="timed launches (default 200; 25 for --impl reference)")
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--workload", default="reachball", choices=["reachball", "shoot", "fullgame"],
@@ -644,16 +670,24 @@ def main():
     ap.add_argument("--cpu-seconds", type=float, default=12.0, help="bound on the cpu_baseline sample")
     ap.add_argument("--no-extras", action="store_true", help="skip the shoot / fullgame sections of the default line")
     ap.add_argument("--no-numa", dest="numa", action="store_false", help="do not bind the rank to its GPU's NUMA node")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed launch as .npy files under DIR (B200 arm)")
     args = ap.parse_args()
+    if args.steps is not None and args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the B200 arm's timed path; use it with --impl b200")
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     if args.impl == "reference":
         args.substeps = args.substeps or SUBSTEPS
-        if args.steps == 200:  # the default K of the B200 arm would take minutes on the CPU: keep it bounded
+        if args.steps is None:  # the default K of the B200 arm would take minutes on the CPU: keep it bounded
             args.steps = 25  # (2.6 s timed)
         run_reference(args, rank)
         return
+    if args.steps is None:
+        args.steps = 200
     if world != args.gpus and world == 1 and args.gpus > 1:
         raise SystemExit(f"--gpus {args.gpus} needs torchrun: python -m torch.distributed.run --nproc-per-node {args.gpus} "
                          f"--master-addr 127.0.0.1 bench.py --gpus {args.gpus} ...")

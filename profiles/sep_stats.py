@@ -1,5 +1,5 @@
 import os, sys
-ROOT = "/root/repo"
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, os.path.join(ROOT, "gym-soccer-2d-env_b200")); sys.path.insert(0, ROOT)
 import torch, bench
 from soccer2d_b200 import Soccer2DVecEnv

@@ -1,110 +1,57 @@
-"""CPU-only: the proto-shaped export (soccer2d_b200.proto_state) parses into the REFERENCE's own generated
-service_pb2.State, and the reference's own ReachBallEnv hooks compute from it what the kernels compute.
-Needs /root/reference (present in the build container, absent on the GPU box -> skipped there)."""
+"""CPU-only: the proto-shaped export (soccer2d_b200.proto_state) is the one the reference's own generated
+service_pb2 parsed and its ReachBall hooks computed from (stored in tests/golden/proto_state.json; with a checkout of
+the reference, tests/golden/make_proto_state.py --reference DIR runs that check again), and the fields those hooks read
+carry what the kernels compute from."""
+import json
 import os
-import sys
 
-import numpy as np
 import pytest
 
-import helpers as H  # noqa: F401  (sys.path)
-from soccer2d_b200 import _abi
-from soccer2d_b200.proto_state import player_type_dict, state_dict, trainer_state_dict
-
-REF = os.environ.get("S2D_REFERENCE", "/root/reference")
-pytestmark = pytest.mark.skipif(not os.path.exists(os.path.join(REF, "service_pb2.py")), reason="reference not mounted")
+import helpers as H
+from golden import make_proto_state as G
+from oracle import soccer2d_oracle as O
+from soccer2d_b200.proto_state import state_dict
 
 
-def _snapshot():
-    s = _abi.EnvSnapshot()
-    s.cycle, s.game_mode_type, s.game_mode_side, s.step_number, s.left_score, s.right_score = 57, 4, 2, 12, 1, 0
-    s.ball_x, s.ball_y, s.ball_vx, s.ball_vy = 10.5, -3.25, 0.5, 0.125
-    s.num_players = 3
-    for j, (x, y, body, side, unum) in enumerate(((-20.0, 4.0, 135.0, 1, 1), (10.0, -3.0, -45.0, 1, 2), (30.0, 0.0, 180.0, 2, 1))):
-        p = s.players[j]
-        p.x, p.y, p.vx, p.vy, p.body_direction = x, y, 0.25, -0.5, body
-        p.stamina, p.effort, p.recovery, p.stamina_capacity, p.side, p.uniform_number = 7500.0, 0.9, 1.0, 120000.0, side, unum
-    return s
+@pytest.fixture(scope="module")
+def stored():
+    with open(os.path.join(H.ROOT, "tests", "golden", "proto_state.json")) as f:
+        return json.load(f)
 
 
-_REF_SIDE = r"""
-import json, logging, sys
-shims, ref, payload = sys.argv[1], sys.argv[2], json.load(sys.stdin)
-sys.path[:0] = [ref, shims]              # the reference's modules + stand-ins for gym / pyrusgeom only
-from google.protobuf import json_format
-import service_pb2 as pb2
-import soccer_2d_env
-soccer_2d_env.Soccer2DEnv.__init__ = lambda self, *a, **k: None      # no rcssserver / proxy processes offline
-from sample_environments.reach_ball_env import ReachBallEnv
-log = logging.getLogger("x"); log.disabled = True
-state = json_format.ParseDict(payload["player"], pb2.State())
-trainer = json_format.ParseDict(payload["trainer"], pb2.State())
-wm = state.world_model
-env = ReachBallEnv(render_mode=None, logger=log, log_dir="/tmp")
-obs = env.state_to_observation(state)
-env.step_number = 5
-done, reward, info = env.check_trainer_observation(trainer)
-print(json.dumps({
-    "cycle": wm.cycle, "mode_is_kick_in": wm.game_mode_type == pb2.GameModeType.KickIn_,
-    "mode_side_is_right": wm.game_mode_side == pb2.Side.RIGHT, "self_unum": wm.self.uniform_number,
-    "self_side_is_left": wm.self.side == pb2.Side.LEFT, "stamina": wm.self.stamina, "n_mates": len(wm.teammates),
-    "n_opps": len(wm.opponents), "left_score": wm.left_team_score, "ball_x": wm.ball.position.x, "ball_vy": wm.ball.velocity.y,
-    "kickable_mate": wm.kickable_teammate_existance, "mate_unum": wm.teammates[0].uniform_number,
-    "type_ids": [wm.self.type_id, wm.teammates[0].type_id, wm.opponents[0].type_id],
-    "our_dict": sorted(wm.our_players_dict), "their_dict": sorted(wm.their_players_dict),
-    "obs": [float(v) for v in obs], "done": bool(done), "reward": float(reward), "result": info["result"]}))
-"""
-
-
-def test_state_dict_parses_into_the_reference_proto_and_feeds_its_hooks():
-    """Runs the reference side in a clean interpreter (its module names - soccer_2d_env, sample_environments - are
-    the same as this repo's host package, on purpose)."""
-    import json
-    import subprocess
-    from oracle import soccer2d_oracle as O
-
-    snap = _snapshot()
-    payload = {"player": state_dict(snap, unum=1, side=1, type_of_player=[0, 7, 3]), "trainer": trainer_state_dict(snap)}
-    r = subprocess.run([sys.executable, "-c", _REF_SIDE, os.path.join(H.ROOT, "tests", "golden", "_shims"), REF],
-                       input=json.dumps(payload), capture_output=True, text=True, env={**os.environ, "PYTHONPATH": ""})
-    assert r.returncode == 0, r.stderr[-2000:]
-    got = json.loads(r.stdout.strip().splitlines()[-1])
-    assert got["cycle"] == 57 and got["mode_is_kick_in"] and got["mode_side_is_right"]
-    assert got["self_unum"] == 1 and got["self_side_is_left"] and got["stamina"] == 7500.0
-    assert (got["n_mates"], got["n_opps"], got["left_score"]) == (1, 1, 1)
-    assert got["ball_x"] == 10.5 and got["ball_vy"] == 0.125
-    assert got["kickable_mate"] and got["mate_unum"] == 2  # player 2 stands next to the ball
-    assert got["our_dict"] == [1, 2] and got["their_dict"] == [1] and got["type_ids"] == [0, 7, 3]
-    # the reference's own observation / reward code on the exported State == the simulator's formulas
-    want = O.build_obs(10.5, -3.25, 0.5, 0.125, -20.0, 4.0, 135.0)
-    assert np.allclose(got["obs"], want, rtol=0, atol=1e-12)
-    d, rw, res, _, _ = O.check_trainer(O.ReachBallConfig(), 0.0, 0.0, 5, 10.5, -3.25, -20.0, 4.0, 135.0)
-    assert (got["done"], got["result"]) == (d, O.RESULT_NAMES[res]) and got["reward"] == pytest.approx(rw, rel=1e-12)
+def test_state_dict_parses_into_the_reference_proto_and_feeds_its_hooks(stored):
+    payload = G.state_payload()
+    assert payload == stored["state"]
+    wm, me = payload["player"]["world_model"], payload["player"]["world_model"]["self"]
+    assert wm["cycle"] == 57 and wm["game_mode_type"] == "KickIn_" and wm["game_mode_side"] == "RIGHT"
+    assert me["uniform_number"] == 1 and me["side"] == "LEFT" and me["stamina"] == 7500.0
+    assert (len(wm["teammates"]), len(wm["opponents"]), wm["left_team_score"]) == (1, 1, 1)
+    assert wm["ball"]["position"]["x"] == 10.5 and wm["ball"]["velocity"]["y"] == 0.125
+    assert wm["kickable_teammate_existance"] and wm["teammates"][0]["uniform_number"] == 2  # player 2 stands next to the ball
+    assert sorted(map(int, wm["our_players_dict"])) == [1, 2] and sorted(map(int, wm["their_players_dict"])) == [1]
+    assert [me["type_id"], wm["teammates"][0]["type_id"], wm["opponents"][0]["type_id"]] == G.TYPE_OF_PLAYER
+    # the fields reach_ball_env.py's state_to_observation / check_trainer_observation read, through the formulas the
+    # reference's hooks are pinned to (tests/golden/reach_ball_contract.json), give what the simulator computes from
+    ball, pos = wm["ball"], me["position"]
+    assert O.build_obs(ball["position"]["x"], ball["position"]["y"], ball["velocity"]["x"], ball["velocity"]["y"],
+                       pos["x"], pos["y"], me["body_direction"]) == O.build_obs(10.5, -3.25, 0.5, 0.125, -20.0, 4.0, 135.0)
+    tw = payload["trainer"]["world_model"]
+    mate = tw["teammates"][0]
+    assert O.check_trainer(O.ReachBallConfig(), 0.0, 0.0, 5, tw["ball"]["position"]["x"], tw["ball"]["position"]["y"],
+                           mate["position"]["x"], mate["position"]["y"], mate["body_direction"]) == \
+        O.check_trainer(O.ReachBallConfig(), 0.0, 0.0, 5, 10.5, -3.25, -20.0, 4.0, 135.0)
     with pytest.raises(ValueError):
-        state_dict(snap, unum=7, side=1)
+        state_dict(G.snapshot(), unum=7, side=1)
 
 
-def test_player_types_parse_into_the_reference_proto():
-    """the drawn player types, exported with the proto's field names, fill the reference's own PlayerType message"""
-    import ctypes as C
-    import json
-    import subprocess
-
-    lib = _abi.load()
-    sp = _abi.ServerParam()
-    assert lib.s2d_default_server_param(C.byref(sp)) == 0
-    types = (_abi.PlayerType * 18)()
-    assert lib.s2d_generate_player_types(5, C.byref(sp), types, 18) == 0
-    payload = [player_type_dict(k, types[k].as_dict(), sp) for k in range(18)]
-    code = ("import json, sys\nsys.path.insert(0, sys.argv[1])\nfrom google.protobuf import json_format\n"
-            "import service_pb2 as pb2\nout = []\n"
-            "for d in json.load(sys.stdin):\n    m = json_format.ParseDict(d, pb2.PlayerType())\n"
-            "    out.append([m.id, m.player_decay, m.kickable_area, m.real_speed_max, m.cycles_to_reach_max_speed])\n"
-            "print(json.dumps(out))\n")
-    r = subprocess.run([sys.executable, "-c", code, REF], input=json.dumps(payload), capture_output=True, text=True,
-                       env={**os.environ, "PYTHONPATH": ""})
-    assert r.returncode == 0, r.stderr[-2000:]
-    got = json.loads(r.stdout.strip().splitlines()[-1])
-    assert [g[0] for g in got] == list(range(18))
-    assert got[0][1] == pytest.approx(0.4) and got[0][2] == pytest.approx(1.085) and got[0][3] == pytest.approx(1.0)
-    assert all(0.95 < g[3] <= 1.05 and 1 <= g[4] < 50 for g in got)
+def test_player_types_parse_into_the_reference_proto(stored):
+    """the drawn player types, exported with the proto's field names, are the PlayerType messages the reference parsed"""
+    types = G.player_types_payload()
+    assert [t["id"] for t in types] == [t["id"] for t in stored["player_types"]] == list(range(18))
+    for got, want in zip(types, stored["player_types"]):
+        assert got.keys() == want.keys()
+        for key, v in want.items():
+            assert got[key] == (v if isinstance(v, int) else pytest.approx(v, rel=1e-12)), (got["id"], key)
+    assert types[0]["player_decay"] == pytest.approx(0.4) and types[0]["kickable_area"] == pytest.approx(1.085)
+    assert types[0]["real_speed_max"] == pytest.approx(1.0)
+    assert all(0.95 < t["real_speed_max"] <= 1.05 and 1 <= t["cycles_to_reach_max_speed"] < 50 for t in types)
