@@ -408,20 +408,31 @@ static cudaError_t launch_step(S2DSim* h, const KernelParams& kp, int k_substeps
     const int64_t nr = static_cast<int64_t>(FgLayout{h->cfg.num_envs, np}.nr());
     const int lpm = h->fg_lanes_per_match > 0 ? h->fg_lanes_per_match : nr <= 49152 ? 2 : 1;
     const int g1 = static_cast<int>(nr / kFgBlock);
-#define S2D_FG(VAR)                                                                                          \
-  do {                                                                                                       \
-    if (lpm == 2) fullgame_step_kernel<VAR, 22, 2><<<g1 * 2, kFgBlock, 0, s>>>(kp, k_substeps, np, ht);      \
-    else fullgame_step_kernel<VAR, 22, 1><<<g1, kFgBlock, 0, s>>>(kp, k_substeps, np, ht);                   \
+// (a non-zero scripted-player mask selects the same kernel with the script compiled in: s2d_scripted.cu)
+#define S2D_FG_GO(VAR, NP, LPM, GRID)                                                                \
+  do {                                                                                               \
+    if (script) {                                                                                    \
+      const cudaError_t e = launch_fullgame_scripted(VAR, NP, LPM, GRID, kp, k_substeps, np, ht, s); \
+      if (e != cudaSuccess) return e;                                                                \
+    }                                                                                                \
+    else fullgame_step_kernel<VAR, NP, LPM><<<GRID, kFgBlock, 0, s>>>(kp, k_substeps, np, ht);       \
   } while (0)
-    if (h->hetero && h->cfg.noise) fullgame_step_kernel<kVarHeteroNoisy, 0, 1><<<g1, kFgBlock, 0, s>>>(kp, k_substeps, np, ht);
-    else if (h->hetero && np == 22) fullgame_step_kernel<kVarHetero, 22, 1><<<g1, kFgBlock, 0, s>>>(kp, k_substeps, np, ht);
-    else if (h->hetero) fullgame_step_kernel<kVarHetero, 0, 1><<<g1, kFgBlock, 0, s>>>(kp, k_substeps, np, ht);
-    else if (h->cfg.noise) fullgame_step_kernel<kVarNoisy, 0, 1><<<g1, kFgBlock, 0, s>>>(kp, k_substeps, np, ht);
+#define S2D_FG(VAR)                                 \
+  do {                                              \
+    if (lpm == 2) S2D_FG_GO(VAR, 22, 2, g1 * 2);    \
+    else S2D_FG_GO(VAR, 22, 1, g1);                 \
+  } while (0)
+    const bool script = kp.scripted_mask != 0u;
+    if (h->hetero && h->cfg.noise) S2D_FG_GO(kVarHeteroNoisy, 0, 1, g1);
+    else if (h->hetero && np == 22) S2D_FG_GO(kVarHetero, 22, 1, g1);
+    else if (h->hetero) S2D_FG_GO(kVarHetero, 0, 1, g1);
+    else if (h->cfg.noise) S2D_FG_GO(kVarNoisy, 0, 1, g1);
     else if (!h->default_sp && np == 22) S2D_FG(kVarRuntime);
-    else if (!h->default_sp) fullgame_step_kernel<kVarRuntime, 0, 1><<<g1, kFgBlock, 0, s>>>(kp, k_substeps, np, ht);
+    else if (!h->default_sp) S2D_FG_GO(kVarRuntime, 0, 1, g1);
     else if (np == 22) S2D_FG(kVarDefault);
-    else fullgame_step_kernel<kVarDefault, 0, 1><<<g1, kFgBlock, 0, s>>>(kp, k_substeps, np, ht);
+    else S2D_FG_GO(kVarDefault, 0, 1, g1);
 #undef S2D_FG
+#undef S2D_FG_GO
   } else if (h->cfg.scenario == S2D_SCENARIO_SHOOT) {
     if (h->cfg.action_mode == S2D_ACT_DISCRETE) S2D_LAUNCH(S2D_SCENARIO_SHOOT, S2D_ACT_DISCRETE);
     else S2D_LAUNCH(S2D_SCENARIO_SHOOT, S2D_ACT_COMMAND);
@@ -840,6 +851,18 @@ static int set_player_types(S2DHandle h, const S2DPlayerType* types, int n, cons
   for (int k = 0; k < S2D_MAX_PIPELINE_SLOTS; ++k)
     if (h->slot_bound[k]) slot_params(h, k);
   h->hetero = true;
+  return S2D_OK;
+}
+
+int s2d_set_scripted_players(S2DHandle h, uint32_t mask) {
+  if (!h) return S2D_ERR_INVALID;
+  if (h->cfg.scenario != S2D_SCENARIO_FULLGAME) return fail(h, S2D_ERR_INVALID, "scripted players exist in FULLGAME only");
+  const int np = s2d_num_players(&h->cfg);
+  if (np < 32 && (mask >> np) != 0u)
+    return fail(h, S2D_ERR_INVALID, "scripted-player mask 0x%x names players beyond the %d of a match", mask, np);
+  h->kp.scripted_mask = mask;  // (the parameter block goes with each launch: the next one enqueued sees it)
+  for (int k = 0; k < S2D_MAX_PIPELINE_SLOTS; ++k)
+    if (h->slot_bound[k]) slot_params(h, k);
   return S2D_OK;
 }
 

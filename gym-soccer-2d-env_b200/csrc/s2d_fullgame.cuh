@@ -131,7 +131,7 @@ __device__ __constant__ float kFgFormY[11] = {0, -20, -7, 7, 20, -24, -8, 8, 24,
 
 // Sum of 32 leaves in xor-butterfly order ((i, i^16), then (i, i^8), ...): leaf i = v[i] where bit i of `mask` is set,
 // else 0.0.  Cold (only cycles with a kick or a ball collision get here), so the leaves live in local memory.
-__device__ __noinline__ float tree_sum32(const float* v, uint32_t mask) {
+__device__ __noinline__ inline float tree_sum32(const float* v, uint32_t mask) {
   float leaf[32];
 #pragma unroll 1
   for (int i = 0; i < 32; ++i) leaf[i] = ((mask >> i) & 1u) ? v[i] : 0.0f;
@@ -158,7 +158,7 @@ __device__ __forceinline__ void fg_place_player(float2& xy, float& body, const K
 }
 
 // every player to its kick-off spot, at rest, facing the opponents (after a goal; cold)
-__device__ __noinline__ void fg_kick_off_formation(FgShared& S, int t, FgPlanes g, const KernelParams& P, uint64_t gid,
+__device__ __noinline__ inline void fg_kick_off_formation(FgShared& S, int t, FgPlanes g, const KernelParams& P, uint64_t gid,
                                                    uint32_t episode, int np, int kick_offs) {
 #pragma unroll 1
   for (int j = 0; j < np; ++j) {
@@ -356,7 +356,7 @@ __device__ __forceinline__ float butterfly_sum(float v) {
 // ball) and the ball in rows 0-4 of its observation staging column (nothing is passed by reference: a variable whose
 // address a non-inlined function has seen lives in local memory for good); the player lanes write positions and velocities back (shared memory, plane PA and,
 // when `obs_rows` (the observation tensor) is set - last cycle of a launch -, the row the player loop has already written).
-__device__ __noinline__ void fg_resolve_collisions(FgShared& S, const int t, const int tid, const int lane, const int lpm, const FgPlanes g,
+__device__ __noinline__ inline void fg_resolve_collisions(FgShared& S, const int t, const int tid, const int lane, const int lpm, const FgPlanes g,
                                                    const float mbx, const float mby, const float mbvx, const float mbvy,
                                                    const int np, unsigned need,
                                                    const bool dead, const float r, const float r2, const int model, float* obs_rows,
@@ -481,7 +481,7 @@ __device__ __noinline__ void fg_resolve_collisions(FgShared& S, const int t, con
 // Offside marks (OffsideRef), taken at the moment of a pass by ONE team in PlayOn: the passer's team-mates that are, in
 // their direction of attack, beyond the ball, the half-way line and the second-last opponent.  Positions are those
 // before the cycle's move (S.oldx, the ball before its move).  Cold: only cycles with a kick.
-__device__ __noinline__ uint32_t fg_offside_marks(const FgShared& S, int t, int np, bool att_left, uint32_t kick_mask, float ball_x) {
+__device__ __noinline__ inline uint32_t fg_offside_marks(const FgShared& S, int t, int np, bool att_left, uint32_t kick_mask, float ball_x) {
   const int pps = np >> 1;
   const float sgn = att_left ? 1.0f : -1.0f;
   const int d0 = att_left ? pps : 0, a0 = att_left ? 0 : pps;
@@ -569,6 +569,94 @@ __device__ __forceinline__ void fg_write_obs(float* __restrict__ dst, int64_t en
   }
 }
 
+// ---- the built-in script (scripted players; spec: include/soccer2d.h, s2d_set_scripted_players) ----
+// A kernel variant: VAR + kVarScripted is the same kernel with the script compiled in; the launcher picks it only when
+// the handle's mask is non-zero, so the kernels without it are the ones that ran before the script existed.
+constexpr int kVarScripted = 8;
+
+// the ball inside the penalty area of the left (right) team
+template <class SP>
+__device__ __forceinline__ bool fg_in_penalty_area(const SP& sp, float bx, float by, bool left) {
+  const float edge = sp.pitch_half_length() - kFgPenaltyLength;
+  return (left ? bx <= -edge : bx >= edge) && fabsf(by) <= kFgPenaltyHalfWidth;
+}
+
+// Chaser of each side: its player nearest to the ball (positions at the start of the cycle, S.xy; ties go to the lower
+// index).  The goalkeeper takes part only while the ball is in its own penalty area, or when it is its side's only player.
+template <class SP>
+__device__ __forceinline__ void fg_script_chasers(const FgShared& S, int t, const SP& sp, const Match& m, int np, int& chaser_l,
+                                                  int& chaser_r) {
+  const int pps = np >> 1;
+  const bool area_l = fg_in_penalty_area(sp, m.bx, m.by, true), area_r = fg_in_penalty_area(sp, m.bx, m.by, false);
+  float best_l = 3.0e38f, best_r = 3.0e38f;
+  chaser_l = chaser_r = -1;
+#pragma unroll 1
+  for (int j = 0; j < np; ++j) {
+    const bool left = j < pps;
+    const bool keeper = j == 0 || j == pps;
+    const bool eligible = !keeper || pps == 1 || (left ? area_l : area_r);
+    const float2 xy = S.xy[j][t];
+    const float dx = xy.x - m.bx, dy = xy.y - m.by;
+    const float d2 = dx * dx + dy * dy;
+    if (eligible && left && d2 < best_l) {
+      best_l = d2;
+      chaser_l = j;
+    }
+    if (eligible && !left && d2 < best_r) {
+      best_r = d2;
+      chaser_r = j;
+    }
+  }
+}
+
+// The command of scripted player j (start-of-cycle position / body in `pa` / `body`, catch bans `ban`), in the rules'
+// order of the spec.  fp32, no contraction, IEEE division and square root (DESIGN.md section 4).
+template <class SP>
+__device__ __forceinline__ float4 fg_script_command(const SP& sp, const Match& m, const float4 pa, const float body, const int j,
+                                                    const int pps, const bool chaser, const uint32_t ban) {
+  const bool left = j < pps;
+  const float sg = left ? 1.0f : -1.0f;  // own frame: (sg x, sg y)
+  const bool keeper = j == 0 || j == pps;
+  const float hl = sp.pitch_half_length(), hw = sp.pitch_half_width();
+  const float post = sp.goal_width() * 0.5f - 1.0f;
+  const float obx = sg * m.bx, oby = sg * m.by;  // the ball in the own frame
+  if (m.mode == S2D_PM_AFTER_GOAL || m.mode == S2D_PM_BEFORE_KICK_OFF || m.mode == S2D_PM_TIME_OVER)
+    return make_float4(static_cast<float>(S2D_CMD_NONE), 0.0f, 0.0f, 0.0f);
+  const bool play_on = m.mode == S2D_PM_PLAY_ON;
+  if (chaser && (play_on || m.side == (left ? S2D_SIDE_LEFT : S2D_SIDE_RIGHT))) {
+    const float dx = m.bx - pa.x, dy = m.by - pa.y;
+    const float d2 = dx * dx + dy * dy;
+    const uint32_t my_ban = j == 0 ? ban & 15u : (ban >> 4) & 15u;
+    if (play_on && keeper && my_ban == 0u && fg_in_penalty_area(sp, m.bx, m.by, left) && d2 <= kFgCatchLength * kFgCatchLength)
+      return make_float4(static_cast<float>(S2D_CMD_CATCH), norm_deg(atan2_deg(dy, dx) - body), 0.0f, 0.0f);
+    if (!(sqrtf(d2) > sp.kickable_area())) {
+      // kick target: within 25 m of the goal centre the far post (seen from the kicker: the ball's side flips while it
+      // is staged around the kicker's feet) at ball_speed_max, else 8 m further towards the goal at 1
+      const float gx = hl - obx, gy = -oby;
+      const float g2 = gx * gx + gy * gy;
+      float tx, ty, speed;
+      if (g2 <= 625.0f) {
+        tx = hl;
+        ty = sg * pa.y >= 0.0f ? -post : post;
+        speed = sp.ball_speed_max();
+      } else {
+        const float k = 8.0f / sqrtf(g2);
+        tx = obx + gx * k;
+        ty = oby + gy * k;
+        speed = 1.0f;
+      }
+      return make_float4(static_cast<float>(S2D_CMD_SMART_KICK), sg * tx, sg * ty, speed);
+    }
+    if (play_on) return make_float4(static_cast<float>(S2D_CMD_INTERCEPT), 0.0f, 0.0f, 0.0f);
+    return make_float4(static_cast<float>(S2D_CMD_GOTO), m.bx, m.by, 100.0f);
+  }
+  if (keeper) return make_float4(static_cast<float>(S2D_CMD_GOTO), sg * (2.5f - hl), sg * clampf(-post, 0.3f * oby, post), 100.0f);
+  const int k = left ? j : j - pps;
+  const float fx = clampf(2.5f - hl, kFgFormX[k] + 0.6f * obx, hl - 2.5f);
+  const float fy = clampf(2.0f - hw, kFgFormY[k] + 0.3f * oby, hw - 2.0f);
+  return make_float4(static_cast<float>(S2D_CMD_GOTO), sg * fx, sg * fy, 60.0f);
+}
+
 // One cycle of the match.  Commands: float4 {cmd, a, b, c} of player j at act[j].  Returns done.
 // `obs_row` != nullptr (last cycle of a launch, 11 v 11): the player loop writes the players' part of the observation
 // row as it goes (the values are in registers then), and whatever moves a player afterwards patches its entry;
@@ -578,7 +666,7 @@ __device__ __forceinline__ void fg_write_obs(float* __restrict__ dst, int64_t en
 // two player loops (sub-lane h takes the groups of four players h, h + LPM, ...) and in the pair scan, merge what they
 // found with shuffles, and repeat the cheap per-match arithmetic (ball, referee) redundantly - bit-identical by
 // construction.  It shortens the dependent chain of a cycle: for shards too small to fill the GPU with one thread per match.
-template <int LPM, class SP>
+template <int LPM, bool SCRIPT, class SP>
 __device__ __forceinline__ bool fg_cycle(FgShared& S, const int t, const int tid, const FgPlanes& g, Match& m, const KernelParams& P,
                                          SP& sp, uint64_t gid, int np, int half_time, const float4* __restrict__ act,
                                          float* obs_row, const bool valid, bool& obs_dirty, float& reward, int& result,
@@ -610,6 +698,11 @@ __device__ __forceinline__ bool fg_cycle(FgShared& S, const int t, const int tid
   float kx[32], ky[32];  // the kickers' pushes on the ball (local memory; written only when somebody kicks)
   float moved2 = 0.0f;
   const uint32_t tk0_in = m.tk0, tk1_in = m.tk1, tk2_in = m.tk2, ban_in = m.ban;
+  int chaser_l = -1, chaser_r = -1;  // scripted players: each side's chaser, from the positions before anybody moves
+  if constexpr (SCRIPT) {
+    fg_script_chasers(S, t, sp, m, np, chaser_l, chaser_r);
+    if (LPM > 1) __syncwarp();  // (the other sub-lanes overwrite S.xy in the player loop)
+  }
   {
     // software pipeline: the plane entries of this sub-lane's next player are in flight while the current one
     // computes; the commands come two players (one 32-byte sector) at a time, so the loop walks the players in pairs
@@ -652,6 +745,10 @@ __device__ __forceinline__ bool fg_cycle(FgShared& S, const int t, const int tid
         prefetch_l2(wpa + (1 + kAhead) * g.row);
         prefetch_l2(wpb + (1 + kAhead) * g.row);
         prefetch_l2(wpc + (1 + kAhead) * g.rowc);
+      }
+      if constexpr (SCRIPT) {  // a scripted player's row of the action buffer is replaced by the script's command
+        if (on && ((P.scripted_mask >> j) & 1u))
+          a = fg_script_command(sp, m, pa, b.x, j, pps, j == (j < pps ? chaser_l : chaser_r), ban_in);
       }
       if (!on) a.x = static_cast<float>(S2D_CMD_NONE);
       const bool left = j < pps;
@@ -1175,7 +1272,8 @@ __global__ void __launch_bounds__(kFgBlock, S2D_FG_MIN_BLOCKS) fullgame_step_ker
                                                                  const int np_runtime, const int half_time) {
   static_assert(LPM == 1 || LPM == 2 || LPM == 4, "lanes per match");
   const int np = NP ? NP : np_runtime;
-  using SP = typename VariantSP<VAR>::type;
+  constexpr bool SCRIPT = (VAR & kVarScripted) != 0;
+  using SP = typename VariantSP<VAR & ~kVarScripted>::type;
   SP sp(P.cc);
   __shared__ FgShared S;
   fg_bind_player_types(sp, P);
@@ -1194,6 +1292,14 @@ __global__ void __launch_bounds__(kFgBlock, S2D_FG_MIN_BLOCKS) fullgame_step_ker
 
   Match m;
   fg_load(P, L, env, m);
+  if constexpr (SCRIPT) {  // the script's chaser pre-pass reads every player's position from shared memory
+#pragma unroll 1
+    for (int j = tid & (LPM - 1); j < np; j += LPM) {
+      const float4 a = ld_stream(g.pa + static_cast<size_t>(j) * g.row);
+      S.xy[j][t] = make_float2(a.x, a.y);
+    }
+    if (LPM > 1) __syncwarp();
+  }
   uint32_t collided_mask = 0, kicked_mask = 0;
   bool ball_collided = false, obs_dirty = false;
   float reward_sum = 0.0f;
@@ -1206,7 +1312,7 @@ __global__ void __launch_bounds__(kFgBlock, S2D_FG_MIN_BLOCKS) fullgame_step_ker
     int rs;
     // in the last cycle of an 11 v 11 launch the player loop writes the observation row itself
     float* const obs_row = (NP == kFgMaxPlayers && k == 1) ? my_obs : nullptr;
-    const bool done = fg_cycle<LPM>(S, t, tid, g, m, P, sp, gid, np, half_time, act, obs_row, valid, obs_dirty, rw, rs, collided_mask,
+    const bool done = fg_cycle<LPM, SCRIPT>(S, t, tid, g, m, P, sp, gid, np, half_time, act, obs_row, valid, obs_dirty, rw, rs, collided_mask,
                                     kicked_mask, ball_collided);
     reward_sum += rw;
     m.ep_return += rw;
@@ -1259,6 +1365,13 @@ __global__ void __launch_bounds__(kFgBlock, S2D_FG_MIN_BLOCKS) fullgame_step_ker
   P.done[env] = static_cast<uint8_t>(any_done);
   P.result[env] = static_cast<uint8_t>(last_result);
 }
+
+// Launches fullgame_step_kernel<var + kVarScripted, np_template, lpm> (s2d_scripted.cu); cudaErrorInvalidValue, and no
+// launch, for a combination it does not instantiate.  The scripted variants live in a
+// translation unit of their own: sharing one with the kernels without the script changed how ptxas compiled the
+// out-of-line functions they have in common, and with them the code of kernels that had not changed.
+cudaError_t launch_fullgame_scripted(int var, int np_template, int lpm, int grid, const KernelParams& kp, int k_substeps,
+                                     int np, int half_time, cudaStream_t s);
 
 template <bool HETERO>
 __global__ void __launch_bounds__(kFgBlock) fullgame_reset_kernel(const __grid_constant__ KernelParams P,

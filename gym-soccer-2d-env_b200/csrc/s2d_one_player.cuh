@@ -395,7 +395,7 @@ __device__ __forceinline__ float2 ball_back_trace(float px, float py, float bx, 
 
 // Ball overlapping the single player (rare): up to ten relaxation rounds as in the server.  MIDPOINT model: the player
 // keeps its place (the average of its proposals is its own position).  The caller applies vel *= -0.1 to both.
-__device__ __noinline__ float2 resolve_ball_player_overlap(float px, float py, float bx, float by, float bvx, float bvy,
+__device__ __noinline__ inline float2 resolve_ball_player_overlap(float px, float py, float bx, float by, float bvx, float bvy,
                                                            float r) {
   const float r2 = r * r;
   const float rr = r + kCollideEps;
@@ -410,7 +410,7 @@ __device__ __noinline__ float2 resolve_ball_player_overlap(float px, float py, f
   return make_float2(bx, by);
 }
 // BACKTRACE model: the player backs up along its own velocity as well.  Returns {ball x, y, player x, y}.
-__device__ __noinline__ float4 resolve_ball_player_overlap_backtrace(float px, float py, float vx, float vy, float bx, float by,
+__device__ __noinline__ inline float4 resolve_ball_player_overlap_backtrace(float px, float py, float vx, float vy, float bx, float by,
                                                                      float bvx, float bvy, float r) {
   const float r2 = r * r;
   const float rr = r + kCollideEps;

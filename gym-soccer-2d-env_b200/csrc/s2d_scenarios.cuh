@@ -41,6 +41,9 @@ struct KernelParams {
   float* terminal_obs;
   unsigned long long* stats;  // [kStatSlots][kStatWords]
   int32_t kick_actions;       // SHOOT Discrete(n): the last kick_actions actions are kicks
+  uint32_t scripted_mask;     // FULLGAME: bit j = player j is played by the built-in script (s2d_set_scripted_players).
+                              // (In the alignment gap before the next pointer: the struct keeps its size and every other
+                              // field and kernel argument its offset in the constant bank.)
   const float* player_types;  // FULLGAME, heterogeneous players: [S2D_MAX_PLAYER_TYPES][PT_ROW] (device), else nullptr
   uint8_t type_of[32];        // player -> row of player_types (one assignment for every match of the handle)
   const uint8_t* type_of_match;  // or one assignment per match: [np][Nr] (device, match-minor like the state), else nullptr

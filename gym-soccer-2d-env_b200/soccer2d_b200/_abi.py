@@ -8,7 +8,7 @@ from __future__ import annotations
 import ctypes as C
 import os
 
-ABI_VERSION = 12
+ABI_VERSION = 13
 MAX_PIPELINE_SLOTS = 4
 
 # ---- constants (mirror include/soccer2d.h) ----------------------------------------------------------
@@ -156,6 +156,7 @@ SIGNATURES = {
     "s2d_generate_player_types": (C.c_int, [C.c_uint64, C.POINTER(ServerParam), C.POINTER(PlayerType), C.c_int]),
     "s2d_set_player_types": (C.c_int, [_H, C.POINTER(PlayerType), C.c_int, C.POINTER(C.c_uint8)]),
     "s2d_set_player_types_per_match": (C.c_int, [_H, C.POINTER(PlayerType), C.c_int, C.POINTER(C.c_uint8)]),
+    "s2d_set_scripted_players": (C.c_int, [_H, C.c_uint32]),
     "s2d_rollout_mlp": (C.c_int, [_H, C.POINTER(MlpPolicy), C.c_int, C.c_float, C.c_void_p, C.c_void_p, C.c_void_p]),
     "s2d_rollout_mlp_collect": (C.c_int, [_H, C.POINTER(MlpPolicy), C.c_int, C.c_float, C.POINTER(Trajectory), C.c_void_p]),
     "s2d_rollout_actor_collect": (C.c_int, [_H, C.POINTER(MlpPolicy), C.c_int, C.c_float, C.POINTER(Trajectory), C.c_void_p]),

@@ -165,6 +165,10 @@ class Soccer2DVecEnv(_VecEnvBase):
     noise          rcssserver's player_rand / ball_rand / kick_rand noise from the counter-based RNG, keyed on
                    (seed, global env id, server cycle, agent): reproducible, independent of sharding and of
                    `substeps`.  Off by default (the mode in which runs are compared with the double-precision CPU truth)
+    scripted_players   fullgame: players played by the built-in script inside the step kernel (include/soccer2d.h,
+                   s2d_set_scripted_players): None (nobody), "left", "right", or an iterable of player indices (left team
+                   first).  Their rows of the action tensor keep their place in its [N, K, players, 4] layout and are
+                   ignored.  The reward stays the left team's view.  See `set_scripted_players`
     collision_model  "midpoint" (default) or "backtrace": which reading of rcssserver's pair rule Stadium::collisions uses
                    (include/soccer2d.h "Collision models"; the binary is not available offline, both are implemented)
     host_numa_node NUMA node for the pinned host staging blocks of step_host / submit_host (soccer2d_b200.numa: the node of
@@ -185,7 +189,7 @@ class Soccer2DVecEnv(_VecEnvBase):
                  env_id_offset: int = 0, auto_reset: bool = True, terminal_obs: bool = False,
                  server_param: dict | None = None, use_command_action: bool = False, goto_dist_thr: float = 0.5,
                  noise: bool = False, host_mapped_io: bool = False, hetero_seed: int | None = None, hetero_per_match: bool = False,
-                 host_numa_node: int | None = None, host_ring: int = 4, collision_model: str = "midpoint", **kwargs):
+                 host_numa_node: int | None = None, host_ring: int = 4, collision_model: str = "midpoint", scripted_players=None, **kwargs):
         if scenario.lower() not in _SCENARIOS:
             raise ValueError(f"Environment {scenario} not found.")  # environment_factory.py:28
         self.scenario = scenario.lower()
@@ -323,6 +327,9 @@ class Soccer2DVecEnv(_VecEnvBase):
                 pick = np.random.default_rng(int(hetero_seed)).integers(1, len(types), size=self.num_players)
                 pick[0] = pick[pps] = 0  # goalkeepers keep the default type, as rcssserver requires
             self.set_player_types(types, pick)
+        self.scripted_players = ()
+        if scripted_players is not None:
+            self.set_scripted_players(scripted_players)
         if _VecEnvBase is not object:
             _VecEnvBase.__init__(self, self.num_envs, self.observation_space, self.action_space)
         self.render_mode = None  # soccer_2d_env.py:36; SB3 reads it with get_attr("render_mode")
@@ -779,6 +786,35 @@ class Soccer2DVecEnv(_VecEnvBase):
         _abi.check(setter(self.handle, arr, len(types), tof.ctypes.data_as(C.POINTER(C.c_uint8))), self.handle)
         self.player_types = [arr[k].as_dict() for k in range(len(types))]
         self.type_of_player = tof.copy()
+
+    # ---- scripted players (fullgame; include/soccer2d.h "FULLGAME scripted players") ------------------------------
+    def scripted_mask(self, players) -> int:
+        """None / "left" / "right" / an iterable of player indices -> the bit mask of s2d_set_scripted_players"""
+        pps = self.num_players // 2
+        if players is None:
+            return 0
+        if isinstance(players, str):
+            if players == "left":
+                return (1 << pps) - 1
+            if players == "right":
+                return ((1 << self.num_players) - 1) & ~((1 << pps) - 1)
+            raise ValueError(f"scripted_players: {players!r} is not 'left', 'right', None or a list of player indices")
+        mask = 0
+        for j in players:
+            j = int(j)
+            if not 0 <= j < self.num_players:
+                raise ValueError(f"scripted_players: player {j} does not exist (0..{self.num_players - 1})")
+            mask |= 1 << j
+        return mask
+
+    def set_scripted_players(self, players) -> None:
+        """Players played by the built-in script from the next step on: None (nobody), "left", "right" or an iterable of
+        player indices (left team first).  Their rows of the action tensor are ignored.  fullgame only (ValueError)."""
+        if self.scenario != "fullgame":
+            raise ValueError("scripted players exist in the fullgame scenario only")
+        mask = self.scripted_mask(players)
+        _abi.check(self.lib.s2d_set_scripted_players(self.handle, mask), self.handle)
+        self.scripted_players = tuple(j for j in range(self.num_players) if (mask >> j) & 1)
 
     def state_dict(self) -> dict:
         return {"state": self.state.clone(), "stats": self.stats_buf.clone(), "seed": self.seed_value,

@@ -42,7 +42,7 @@
 extern "C" {
 #endif
 
-#define S2D_ABI_VERSION 12
+#define S2D_ABI_VERSION 13
 
 /* error codes */
 #define S2D_OK 0
@@ -127,6 +127,40 @@ extern "C" {
  *   xor butterfly ((i, i^16), (i, i^8), ... ; leaf = player index, the others 0.0): part of the fp32 result.
  *   State buffer: s2d_state_bytes(cfg) = Nr * (np * 36 + 80) bytes, Nr = N rounded up to 64; plane-major, match-minor
  *   (layout: DESIGN.md). */
+
+/* FULLGAME scripted players (s2d_set_scripted_players; not in the reference - this is the spec).  One fixed baseline team
+ * that runs inside the step kernel, so that a team, or one player, can be trained against it without writing the others.
+ * Bit j of the handle's mask set: player j (left team first) plays by the rules below and its row of the action buffer
+ * is ignored.  Mask 0 (the default): nothing changes.  The script's command then goes through the cycle exactly as a
+ * command from the action buffer would (catch ban, tackle counters, kick-off confinement, dead-ball clearance).
+ *   Inputs: the state at the START of the cycle - the ball, the player's own position, velocity, body and catch ban, the
+ *   play mode and its side, and the other players' positions only.  No randomness.  fp32 arithmetic as the rest of the cycle.
+ *   Notation: sg = +1 for the left team, -1 for the right; own frame (sg x, sg y) (the point reflection of the kick-off
+ *   formation); L = pitch_half_length, W = pitch_half_width, P = goal_width / 2 - 1; F_k = the kick-off spot of team slot k
+ *   (left-team coordinates, 4-4-2: (-50, 0) (-36, -20) (-36, -7) (-36, 7) (-36, 20) (-20, -24) (-20, -8) (-20, 8)
+ *   (-20, 24) (-9, -10) (-9, 10)); b' = (bx', by') = the ball in the own frame; clamp(v, a) = max(-a, min(v, a));
+ *   d2 = dx * dx + dy * dy with (dx, dy) = ball - player; "in the penalty area" as for catch (|x| >= L - 16.5 on the own
+ *   side, |y| <= 20.16).
+ *   Chaser of each side (decided once per cycle, before anybody moves): the side's player with the smallest d2, ties to
+ *   the lower index.  The goalkeeper (player 0 / players_per_side) takes part only while the ball is in its own penalty
+ *   area, or when it is its side's only player.
+ *   Kick target T (own frame): gx = L - bx', gy = -by', g2 = gx * gx + gy * gy.
+ *     g2 <= 625 (within 25 m of the goal centre): shoot at the far post as seen from the kicker, T = (L, py' >= 0 ? -P : P)
+ *       (py' = the kicker's own-frame y: the ball's own side of the goal flips back and forth while a kick is staged
+ *       around the kicker's feet), first speed ball_speed_max;
+ *     else dribble: k = 8 / sqrt(g2), T = (bx' + gx * k, by' + gy * k), first speed 1.
+ *   Rules for scripted player j of side s, the first that applies:
+ *     1. play mode AfterGoal, BeforeKickOff or TimeOver: NONE.
+ *     2. j is s's chaser and the mode is PlayOn or a dead ball for s:
+ *        a. PlayOn, j is the goalkeeper, its catch ban is 0, the ball is in its penalty area and d2 <= 1.2 * 1.2:
+ *           CATCH(norm_deg(atan2(dy, dx) - body)) (degrees, -180..180);
+ *        b. else sqrt(d2) <= kickable_area (of j's player type): SMART_KICK(sg T, first speed);
+ *        c. else PlayOn: INTERCEPT;
+ *        d. else (dead ball for s): GOTO(ball, max_dash_power 100).
+ *     3. j is the goalkeeper: GOTO(sg (2.5 - L, clamp(0.3 by', P)), 100).
+ *     4. everybody else: GOTO(sg (clamp(F_k.x + 0.6 bx', L - 2.5), clamp(F_k.y + 0.3 by', W - 2)), 60).
+ *   It does not pass, tackle, mark, or use stamina wisely; it is a baseline, not helios-base.  Two scripted teams against
+ *   each other score little (the two chasers kick the ball into each other: profiles/README.md). */
 
 /* action encodings (reach_ball_env.py:39-47, :53-85) */
 #define S2D_ACT_DISCRETE 0   /* uint8  [N][K]      Discrete(n): Dash(100, (a*360/n)%360-180) (+ kicks in SHOOT)  */
@@ -413,6 +447,12 @@ int s2d_set_player_types(S2DHandle h, const S2DPlayerType* types, int n, const u
  * device copy (num_players bytes per match, read once per player and cycle).  The type TABLE stays one per handle: the
  * matches differ in who plays with which of the n types, not in the types themselves. */
 int s2d_set_player_types_per_match(S2DHandle h, const S2DPlayerType* types, int n, const uint8_t* type_of_player);
+
+/* FULLGAME: the players played by the built-in script (spec above): bit j = player j, left team first; bits >= s2d_num_players
+ * are rejected (S2D_ERR_INVALID), as is any other scenario.  0 = none (the default).  Takes effect from the next launch
+ * enqueued (s2d_step, s2d_step_host, s2d_submit_host); with a non-zero mask the step runs a variant of the kernel with
+ * the script compiled in. */
+int s2d_set_scripted_players(S2DHandle h, uint32_t mask);
 
 /* Closed-loop rollout with the policy inside the kernel (S2D_ACT_DISCRETE; REACHBALL with at most 16 actions, SHOOT
  * with at most 24).
