@@ -101,9 +101,13 @@ S2D_HD void dash_direction(float dir, const SP& sp, float& snapped, float& rate)
 
 // The episode half: stamina is charged first, then the effective power is scaled by effort, the rate and
 // dash_power_rate.  Gives the player's acceleration (it is the only contribution in a cycle).
+// memo_direct (a compile-time constant at the call site): sincos_memo is set and the caller knows that body and
+// direction are whole degrees in [-180, 180] and the dash is not a back dash (step_kernel, ReachBall Discrete(n)), so
+// their sum indexes the memo without the per-cycle test.
 template <class SP>
 __device__ __forceinline__ void dash_apply(Episode& e, float power, float dir, float rate, const SP& sp, float& ax,
-                                           float& ay, bool left_team = true, const float2* sincos_memo = nullptr) {
+                                           float& ay, bool left_team = true, const float2* sincos_memo = nullptr,
+                                           bool memo_direct = false) {
   power = clampf(sp.min_dash_power(), power, sp.max_dash_power());
   const bool back = power < 0.0f;
   float need = back ? power * -2.0f : power;
@@ -115,8 +119,15 @@ __device__ __forceinline__ void dash_apply(Episode& e, float power, float dir, f
   if (slow != 1.0f && e.py < 0.0f) eff = cold_div(eff, slow);
   dir = back ? dir + 180.0f : dir;
   float s, c;
-  if (sincos_memo) sincos_deg_memo(e.body + dir, sincos_memo, s, c);  // the same bits, see s2d_math.cuh
-  else sincos_deg(e.body + dir, s, c);
+  if (memo_direct) {
+    const float2 t = __ldg(sincos_memo + (static_cast<int>(e.body + dir) + kSinCosMemoHalf));
+    s = t.x;
+    c = t.y;
+  } else if (sincos_memo) {
+    sincos_deg_memo(e.body + dir, sincos_memo, s, c);  // the same bits, see s2d_math.cuh
+  } else {
+    sincos_deg(e.body + dir, s, c);
+  }
   ax = eff * c;
   ay = eff * s;
 }
@@ -336,11 +347,8 @@ __device__ __forceinline__ void decode_command(const Episode& e, float4 a, float
 
 // MPObject::_inc.  The two clamps compare SQUARED lengths (no square root unless a clamp applies).
 // NOISE: vel += (U(-m, m), U(-m, m)) with m = rnd * |vel|, drawn for `agent`.
-template <bool NOISE = false>
-__device__ __forceinline__ void move_object(float& x, float& y, float& vx, float& vy, float ax, float ay,
-                                            float accel_max, float accel_max2, float speed_max, float speed_max2,
-                                            float decay, float rnd = 0.0f, const NoiseCtx* nz = nullptr,
-                                            uint32_t agent = 0) {
+__device__ __forceinline__ void accelerate(float& vx, float& vy, float ax, float ay, float accel_max, float accel_max2,
+                                           float speed_max, float speed_max2) {
   if (ax != 0.0f || ay != 0.0f) {
     const float a2 = ax * ax + ay * ay;
     if (a2 > accel_max2) {
@@ -357,12 +365,49 @@ __device__ __forceinline__ void move_object(float& x, float& y, float& vx, float
       vy *= k;
     }
   }
+}
+__device__ __noinline__ inline float2 cold_accelerate(float vx, float vy, float ax, float ay, float accel_max,
+                                                      float accel_max2, float speed_max, float speed_max2) {
+  accelerate(vx, vy, ax, ay, accel_max, accel_max2, speed_max, speed_max2);
+  return make_float2(vx, vy);
+}
+
+template <bool NOISE = false>
+__device__ __forceinline__ void move_object(float& x, float& y, float& vx, float& vy, float ax, float ay,
+                                            float accel_max, float accel_max2, float speed_max, float speed_max2,
+                                            float decay, float rnd = 0.0f, const NoiseCtx* nz = nullptr,
+                                            uint32_t agent = 0) {
+  accelerate(vx, vy, ax, ay, accel_max, accel_max2, speed_max, speed_max2);
   if (NOISE) {
     const uint4 w = noise_block(*nz, agent);
     const float m = rnd * hypot2(vx, vy);
     vx += m * u11(w.x);
     vy += m * u11(w.y);
   }
+  x += vx;
+  y += vy;
+  vx *= decay;
+  vy *= decay;
+}
+
+// move_object (without noise) for a dashing player, in straight-line code: the usual dash is a non-zero acceleration
+// that neither clamp touches (under the default ServerParam, |a| <= 100 * 0.006 < 1 and the speed settles at
+// 0.6 / (1 - 0.4) < 1.05).  The sums and squared lengths are formed up front - the same operations in the same order -
+// and one test sends a clamp, or a zero acceleration (adding it would turn a velocity component of -0 into +0), to
+// move_object's own sequence out of line.
+__device__ __forceinline__ void move_dashing(float& x, float& y, float& vx, float& vy, float ax, float ay,
+                                             float accel_max, float accel_max2, float speed_max, float speed_max2,
+                                             float decay) {
+  const float a2 = ax * ax + ay * ay;
+  float wx = vx + ax, wy = vy + ay;
+  const float v2 = wx * wx + wy * wy;
+  if ((ax == 0.0f && ay == 0.0f) || a2 > accel_max2 || v2 > speed_max2) {
+    const float2 w = cold_accelerate(vx, vy, ax, ay, accel_max, accel_max2, speed_max, speed_max2);
+    wx = w.x;
+    wy = w.y;
+  }
+  vx = wx;
+  vy = wy;
   x += vx;
   y += vy;
   vx *= decay;
@@ -488,19 +533,23 @@ __device__ __forceinline__ void update_stamina(Episode& e, const SP& sp) {
 template <bool TURNS, bool KICKS, class SP>
 __device__ __forceinline__ void simulate_cycle(Episode& e, int cmd, float power, float dir, float rate, const SP& sp,
                                                float& dx, float& dy, float& d2, uint64_t seed, uint64_t gid,
-                                               const float2* sincos_memo = nullptr) {
+                                               const float2* sincos_memo = nullptr, bool memo_direct = false) {
   float ax = 0.0f, ay = 0.0f, bax = 0.0f, bay = 0.0f;
   const NoiseCtx nz{seed, gid, e.cycle};
   if (KICKS) e.flags &= ~S2D_FLAG_KICKED;
   if (cmd == S2D_CMD_DASH) {
-    dash_apply(e, power, dir, rate, sp, ax, ay, true, sincos_memo);
+    dash_apply(e, power, dir, rate, sp, ax, ay, true, sincos_memo, memo_direct);
   } else if (TURNS && cmd == S2D_CMD_TURN) {
     turn(e, dir, sp, nz);
   } else if (KICKS && cmd == S2D_CMD_KICK) {
     if (kick(e, power, dir, sp, bax, bay, nz)) e.flags |= S2D_FLAG_KICKED;
   }
-  move_object<SP::kNoise>(e.px, e.py, e.vx, e.vy, ax, ay, sp.player_accel_max(), sp.player_accel_max2(),
-                          sp.player_speed_max(), sp.player_speed_max2(), sp.player_decay(), sp.player_rand(), &nz, 0u);
+  if (!SP::kNoise && cmd == S2D_CMD_DASH)
+    move_dashing(e.px, e.py, e.vx, e.vy, ax, ay, sp.player_accel_max(), sp.player_accel_max2(), sp.player_speed_max(),
+                 sp.player_speed_max2(), sp.player_decay());
+  else
+    move_object<SP::kNoise>(e.px, e.py, e.vx, e.vy, ax, ay, sp.player_accel_max(), sp.player_accel_max2(),
+                            sp.player_speed_max(), sp.player_speed_max2(), sp.player_decay(), sp.player_rand(), &nz, 0u);
   move_object<SP::kNoise>(e.bx, e.by, e.bvx, e.bvy, bax, bay, sp.ball_accel_max(), sp.ball_accel_max2(),
                           sp.ball_speed_max(), sp.ball_speed_max2(), sp.ball_decay(), sp.ball_rand(), &nz, kBallAgent);
   dx = e.bx - e.px;

@@ -31,6 +31,9 @@ struct KernelParams {
   float min_distance_to_ball, ball_position_x, ball_position_y, ball_speed, ball_direction;
   float travel_factor;  // (1 - 0.96^max_steps) / (1 - 0.96), reach_ball_env.py:207
   float goto_dist_thr;
+  int32_t dash_dirs_whole;  // Discrete(n): every dash of action_table has a whole-degree direction in [-180, 180] and
+                            // is not a back dash, so body + direction of a whole-degree body is a memo index
+                            // (in the alignment gap before `state`, like scripted_mask below)
   // device buffers (caller-owned, see S2DBuffers)
   void* state;
   const void* actions;
@@ -84,11 +87,14 @@ inline void make_kernel_params(const S2DConfig& cfg, KernelParams& kp, float4 ta
   auto direction = [](int a, int n) {
     return n > 0 ? static_cast<float>(fmod(static_cast<double>(a) * 360.0 / static_cast<double>(n), 360.0) - 180.0) : 0.0f;
   };
+  // dash_apply turns Dash(100, .) into a back dash when max_dash_power < 0
+  kp.dash_dirs_whole = fmaxf(sp.min_dash_power(), fminf(100.0f, sp.max_dash_power())) >= 0.0f;
   for (int a = 0; a < 256; ++a) {
     if (a < n_dash || kp.kick_actions == 0) {
       table[a].x = static_cast<float>(S2D_CMD_DASH);
       table[a].y = 100.0f;
       dash_direction(direction(a, n_dash), sp, table[a].z, table[a].w);
+      kp.dash_dirs_whole = kp.dash_dirs_whole && rintf(table[a].z) == table[a].z && fabsf(table[a].z) <= 180.0f;
     } else {
       table[a] = make_float4(static_cast<float>(S2D_CMD_KICK), 100.0f, direction(a - n_dash, kp.kick_actions), 0.0f);
     }
@@ -125,10 +131,25 @@ struct LaunchOut {
 // order Goal -> Out -> Timeout; leaving the pitch ADDS 10 (`reward -= -10.0`, :144).
 // body, mem_ang and atan2's result are already in [-180, 180], so AngleDeg's re-normalisations are identities.
 // (dx, dy) = ball - player and d2 = dx*dx + dy*dy as left by simulate_cycle.
+// Ball and player a few micrometres to a million metres apart (every state an episode reaches, collisions included:
+// a resolved overlap leaves them collide_r apart) take the square root and atan2's division without the IEEE range
+// guards (s2d_math.cuh, in_range_vector); anything else, such as coincident centres or a component below 2^-100 m,
+// takes the IEEE operators out of line.
+__device__ __noinline__ inline float2 cold_dist_angle(float dx, float dy, float d2) {
+  return make_float2(sqrtf(d2), atan2_deg(dy, dx));
+}
 __device__ __forceinline__ bool check_episode(Episode& e, const KernelParams& P, float dx, float dy, float d2,
                                               float& reward, int& result) {
-  const float dist = sqrtf(d2);
-  const float diff = norm_deg_360(atan2_deg(dy, dx) - e.body);
+  float dist, th;
+  if (in_range_vector(dx, dy, d2)) {
+    dist = sqrt_in_range(d2);
+    th = atan2_deg<true>(dy, dx);
+  } else {
+    const float2 c = cold_dist_angle(dx, dy, d2);
+    dist = c.x;
+    th = c.y;
+  }
+  const float diff = norm_deg_360(th - e.body);
   float rw = e.mem_dist - dist;
   rw += (fabsf(e.mem_ang) - fabsf(diff)) * static_cast<float>(1.0 / 180.0);
   const bool goal = dist < P.min_distance_to_ball;
@@ -387,7 +408,7 @@ __device__ __forceinline__ void reset_episode(Episode& e, const KernelParams& P,
 template <int SCN, int ACT, class SP, bool DEFER_END = false>
 __device__ __forceinline__ int substep(Episode& e, const KernelParams& P, const SP& sp, uint64_t gid, int64_t i, float a0,
                                         float a1, float a2, float a3, LaunchOut& out,
-                                        const float2* sincos_memo = nullptr) {
+                                        const float2* sincos_memo = nullptr, bool memo_direct = false) {
   constexpr bool kTurns = ACT == S2D_ACT_TURNING || ACT == S2D_ACT_COMMAND;
   constexpr bool kKicks = ACT == S2D_ACT_COMMAND || SCN == S2D_SCENARIO_SHOOT;
   e.step_number += 1;  // reach_ball_env.py:55
@@ -417,7 +438,7 @@ __device__ __forceinline__ int substep(Episode& e, const KernelParams& P, const 
   float dx, dy, d2, rw;
   int rs;
   const float pbx = e.bx, pby = e.by;
-  simulate_cycle<kTurns, kKicks>(e, cmd, power, dir, rate, sp, dx, dy, d2, P.seed, gid, sincos_memo);
+  simulate_cycle<kTurns, kKicks>(e, cmd, power, dir, rate, sp, dx, dy, d2, P.seed, gid, sincos_memo, memo_direct);
   const bool done = scenario_check<SCN>(e, P, sp, dx, dy, d2, pbx, pby, rw, rs);
   out.reward_sum += rw;
   e.ep_return += rw;
@@ -606,20 +627,30 @@ __global__ void __launch_bounds__(kBlock, S2D_MIN_BLOCKS) step_kernel(const __gr
     // the dash's sin / cos come from the memo (s2d_math.cuh; 5.8 KB, it stays in L1 next to the action table) when
     // the launch is long enough for that to matter.
     const float2* memo = (SCN != S2D_SCENARIO_SHOOT && K >= kSinCosMemoMinK) ? P.sincos_memo : nullptr;
-    // the 4 KB action table stays in L1 (read-only path); `act` walks the lane's K action bytes
-    const uint8_t* act = static_cast<const uint8_t*>(P.actions) + il * K;
+    // When the table's directions and every body of the warp are whole degrees in [-180, 180], body + direction is the
+    // memo index itself, for the whole launch: a new episode's body is a whole degree too (draw_placement).  A body
+    // imported off that grid keeps its warp on sincos_deg_memo's per-cycle test until the next launch.
+    // The K loop is compiled twice, so that the choice costs nothing per cycle.
+    const bool memo_direct = memo && P.dash_dirs_whole &&
+                             __all_sync(0xffffffffu, rintf(e.body) == e.body && fabsf(e.body) <= 180.0f);
+    auto k_loop = [&](auto direct) {
+      // the 4 KB action table stays in L1 (read-only path); `act` walks the lane's K action bytes
+      const uint8_t* act = static_cast<const uint8_t*>(P.actions) + il * K;
 #pragma unroll 1
-    for (int k = K; k > 0; --k, ++act) {
-      int rs;
-      if (SCN == S2D_SCENARIO_SHOOT) {
-        const float4 t = __ldg(P.action_table + __ldg(act));
-        rs = substep<SCN, ACT, SP, true>(e, P, sp, gid, i, t.x, t.y, t.z, t.w, out);
-      } else {  // ReachBall: always Dash(100, .): only the lowered direction and its rate are needed
-        const float2 t = __ldg(reinterpret_cast<const float2*>(P.action_table + __ldg(act)) + 1);
-        rs = substep<SCN, ACT, SP, true>(e, P, sp, gid, i, 0.f, 0.f, t.x, t.y, out, memo);
+      for (int k = K; k > 0; --k, ++act) {
+        int rs;
+        if (SCN == S2D_SCENARIO_SHOOT) {
+          const float4 t = __ldg(P.action_table + __ldg(act));
+          rs = substep<SCN, ACT, SP, true>(e, P, sp, gid, i, t.x, t.y, t.z, t.w, out);
+        } else {  // ReachBall: always Dash(100, .): only the lowered direction and its rate are needed
+          const float2 t = __ldg(reinterpret_cast<const float2*>(P.action_table + __ldg(act)) + 1);
+          rs = substep<SCN, ACT, SP, true>(e, P, sp, gid, i, 0.f, 0.f, t.x, t.y, out, memo, decltype(direct)::value);
+        }
+        end_of_episode<SCN>(e, P, sp, gid, i, valid, rs, out);
       }
-      end_of_episode<SCN>(e, P, sp, gid, i, valid, rs, out);
-    }
+    };
+    if (SCN != S2D_SCENARIO_SHOOT && memo_direct) k_loop(std::true_type());
+    else k_loop(std::false_type());
   } else if (ACT == S2D_ACT_CONTINUOUS) {
     // Box(1): the direction a * 180 is snapped to dash_angle_step = 1 as well and nobody turns - whole degrees again
     const float2* memo = K >= kSinCosMemoMinK ? P.sincos_memo : nullptr;
