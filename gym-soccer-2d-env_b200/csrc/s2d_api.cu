@@ -148,7 +148,8 @@ static bool config_ok(const S2DConfig* c, char* why, size_t n) {
   const bool mode_ok = c->scenario == S2D_SCENARIO_FULLGAME
                            ? c->action_mode == S2D_ACT_COMMAND
                            : c->scenario == S2D_SCENARIO_SHOOT
-                                 ? (c->action_mode == S2D_ACT_DISCRETE || c->action_mode == S2D_ACT_COMMAND)
+                                 ? (c->action_mode == S2D_ACT_DISCRETE || c->action_mode == S2D_ACT_COMMAND ||
+                                    c->action_mode == S2D_ACT_PARAMETERIZED)
                                  : (c->action_mode >= S2D_ACT_DISCRETE && c->action_mode <= S2D_ACT_COMMAND);
   if (!mode_ok) {
     snprintf(why, n, "action_mode %d is not valid for scenario %d", c->action_mode, c->scenario);
@@ -176,6 +177,7 @@ static size_t action_elem_bytes(const S2DConfig* c) {
     case S2D_ACT_DISCRETE: return 1;
     case S2D_ACT_CONTINUOUS: return 4;
     case S2D_ACT_TURNING: return 16;
+    case S2D_ACT_PARAMETERIZED: return 32;
     default: return 16 * static_cast<size_t>(s2d_num_players(c));
   }
 }
@@ -434,7 +436,12 @@ static cudaError_t launch_step(S2DSim* h, const KernelParams& kp, int k_substeps
 #undef S2D_FG
 #undef S2D_FG_GO
   } else if (h->cfg.scenario == S2D_SCENARIO_SHOOT) {
-    if (h->cfg.action_mode == S2D_ACT_DISCRETE) S2D_LAUNCH(S2D_SCENARIO_SHOOT, S2D_ACT_DISCRETE);
+    if (h->cfg.action_mode == S2D_ACT_PARAMETERIZED) {  // (s2d_shoot_param.cu)
+      const int var = h->cfg.noise ? kVarNoisy : h->default_sp ? kVarDefault : kVarRuntime;
+      const cudaError_t e = launch_shoot_param(var, h->grid, kp, k_substeps, s);
+      if (e != cudaSuccess) return e;
+    }
+    else if (h->cfg.action_mode == S2D_ACT_DISCRETE) S2D_LAUNCH(S2D_SCENARIO_SHOOT, S2D_ACT_DISCRETE);
     else S2D_LAUNCH(S2D_SCENARIO_SHOOT, S2D_ACT_COMMAND);
   } else {
     switch (h->cfg.action_mode) {
@@ -879,9 +886,17 @@ static int rollout_mlp(S2DHandle h, const S2DMlpPolicy* policy, int k_substeps, 
   if (!h->bound) return fail(h, S2D_ERR_UNBOUND, "s2d_bind has not been called");
   const bool shoot = h->cfg.scenario == S2D_SCENARIO_SHOOT;
   const int mode = h->cfg.action_mode;
-  if (actor) {
+  const bool param = actor && shoot && mode == S2D_ACT_PARAMETERIZED;
+  if (actor && !param) {
     if (h->cfg.scenario != S2D_SCENARIO_REACHBALL || (mode != S2D_ACT_CONTINUOUS && mode != S2D_ACT_TURNING))
-      return fail(h, S2D_ERR_INVALID, "s2d_rollout_actor_collect: REACHBALL with Box(1) or Box(4) actions only");
+      return fail(h, S2D_ERR_INVALID,
+                  "s2d_rollout_actor_collect: REACHBALL with Box(1) or Box(4) actions, or SHOOT with parameterized actions only");
+  } else if (actor) {
+    // the mma.sync kernels are kept as a measured comparison for the existing spaces only
+    if (policy && policy->precision != 0)
+      return fail(h, S2D_ERR_INVALID, "s2d_rollout_actor_collect: SHOOT parameterized actions need precision 0 (TF32, tcgen05)");
+    if (reinterpret_cast<uintptr_t>(traj.actions_f) & 15)
+      return fail(h, S2D_ERR_INVALID, "s2d_rollout_actor_collect: actions_f must be 16-byte aligned (32-byte rows)");
   } else if (h->cfg.scenario == S2D_SCENARIO_FULLGAME || mode != S2D_ACT_DISCRETE || h->cfg.action_space_size > (shoot ? 24 : 16)) {
     return fail(h, S2D_ERR_INVALID, "s2d_rollout_mlp: REACHBALL with Discrete(n <= 16) or SHOOT with Discrete(n <= 24) actions only");
   }
@@ -890,7 +905,7 @@ static int rollout_mlp(S2DHandle h, const S2DMlpPolicy* policy, int k_substeps, 
   if (k_substeps < 1 || k_substeps > kMaxSubsteps) return fail(h, S2D_ERR_INVALID, "k_substeps must be in 1..%d", kMaxSubsteps);
   if (!(epsilon >= 0.0f && epsilon <= 1.0f)) return fail(h, S2D_ERR_INVALID, "epsilon / noise must be in [0, 1]");
   DeviceGuard guard(h->cfg.device);
-  const int outputs = actor ? (mode == S2D_ACT_TURNING ? 4 : 1) : h->cfg.action_space_size;
+  const int outputs = actor ? (param ? 8 : mode == S2D_ACT_TURNING ? 4 : 1) : h->cfg.action_space_size;
   const MlpWeights w{policy->w1, policy->b1, policy->w2, policy->b2, policy->w3, policy->b3, kObsDim, outputs};
   cudaStream_t s = static_cast<cudaStream_t>(stream);
   if (int rc = before_user_op(h, s)) return rc;
@@ -904,6 +919,13 @@ static int rollout_mlp(S2DHandle h, const S2DMlpPolicy* policy, int k_substeps, 
   } while (0)
   if (policy->precision < 0 || policy->precision > 2)
     return fail(h, S2D_ERR_INVALID, "precision: 0 (TF32, tcgen05), 1 (bf16, mma.sync), 2 (TF32, mma.sync)");
+  if (param) {  // (s2d_shoot_param.cu)
+    const int var = h->cfg.noise ? kVarNoisy : h->default_sp ? kVarDefault : kVarRuntime;
+    S2D_CUDA(h, launch_shoot_param_actor(var, h->grid, h->kp, k_substeps, w, epsilon, traj, s));
+    S2D_CUDA(h, cudaGetLastError());
+    h->env_steps += static_cast<uint64_t>(h->cfg.num_envs) * static_cast<uint64_t>(k_substeps);
+    return after_user_op(h, s);
+  }
   if (policy->precision == 0) {  // the network on tcgen05 (TF32 operands, accumulators in tensor memory)
 #define S2D_TC5(SCN, ACT)                                                                                              \
   do {                                                                                                                 \

@@ -167,15 +167,17 @@ __device__ __forceinline__ void tc5_hidden_epilogue(uint32_t d_tmem, uint32_t a_
 // K closed-loop cycles (observe, network on tcgen05, action, step) of a one-player scenario: the same contract as
 // rollout_mlp_kernel<SCN, VAR, ACT>.  ACT = S2D_ACT_DISCRETE: W is a Q-network, (epsilon-)greedy action.
 // ACT = S2D_ACT_CONTINUOUS / S2D_ACT_TURNING (ReachBall): W is a DDPG actor - tanh of the last layer's first 1 / 4 outputs is
-// the Box(1) / Box(4) action, `epsilon` the half-width of the uniform exploration noise.
+// the Box(1) / Box(4) action, `epsilon` the half-width of the uniform exploration noise.  ACT = S2D_ACT_PARAMETERIZED
+// (Shoot, s2d_shoot_param.cu): the first 8 outputs, translated to the command row the step kernel would make of them.
 template <int SCN, int VAR, int ACT = S2D_ACT_DISCRETE>
 __global__ void __launch_bounds__(kBlock, S2D_ROLLOUT_MIN_BLOCKS)
     rollout_mlp_tc5_kernel(const __grid_constant__ KernelParams P, const int K, const MlpWeights W, const float epsilon,
                            uint8_t* __restrict__ actions_out, float* __restrict__ q_out, const TrajOut T) {
   static_assert(kBlock == 128, "one block = one M = 128 tile");
   constexpr bool kActor = ACT != S2D_ACT_DISCRETE;
-  constexpr int kActDim = ACT == S2D_ACT_TURNING ? 4 : 1;
-  constexpr int N3 = SCN == S2D_SCENARIO_SHOOT ? 32 : 16;  // layer 3's N (a multiple of 16); q_out rows hold 8 NT values
+  constexpr int kActDim = ACT == S2D_ACT_TURNING ? 4 : ACT == S2D_ACT_PARAMETERIZED ? 8 : 1;
+  // layer 3's N (a multiple of 16): 32 for Shoot's 24 Q-values, else 16; q_out rows hold 8 NT values
+  constexpr int N3 = SCN == S2D_SCENARIO_SHOOT && !kActor ? 32 : 16;
   constexpr int NQ = SCN == S2D_SCENARIO_SHOOT ? 24 : 16;
   using SP = typename VariantSP<VAR>::type;
   const SP sp(P.cc);
@@ -253,14 +255,21 @@ __global__ void __launch_bounds__(kBlock, S2D_ROLLOUT_MIN_BLOCKS)
     // the thread's own output row.  Q-network: + bias, first maximum wins (as torch.argmax); actor: tanh(. + bias)
     int a = 0;
     float4 av = make_float4(0.0f, 0.0f, 0.0f, 0.0f);
+    float4 av2 = make_float4(0.0f, 0.0f, 0.0f, 0.0f);  // components 4..7 (S2D_ACT_PARAMETERIZED)
     if (kActor) {
       float v[16];
       tc5_ld16(rd, v);
       av.x = tanh_poly(v[0] + s.b3[0]);
-      if (kActDim == 4) {
+      if (kActDim >= 4) {
         av.y = tanh_poly(v[1] + s.b3[1]);
         av.z = tanh_poly(v[2] + s.b3[2]);
         av.w = tanh_poly(v[3] + s.b3[3]);
+      }
+      if constexpr (kActDim == 8) {
+        av2.x = tanh_poly(v[4] + s.b3[4]);
+        av2.y = tanh_poly(v[5] + s.b3[5]);
+        av2.z = tanh_poly(v[6] + s.b3[6]);
+        av2.w = tanh_poly(v[7] + s.b3[7]);
       }
     } else {
       float best = -3.4e38f;
@@ -295,7 +304,24 @@ __global__ void __launch_bounds__(kBlock, S2D_ROLLOUT_MIN_BLOCKS)
         av.y = clampf(-1.0f, av.y + epsilon * u11(w.y), 1.0f);
         av.z = clampf(-1.0f, av.z + epsilon * u11(w.z), 1.0f);
         av.w = clampf(-1.0f, av.w + epsilon * u11(w.w), 1.0f);
+        if constexpr (kActDim == 8) {  // (counter 3 of RNG_ACTION: drawn by nothing else)
+          const uint4 w2 = philox4x32_10(P.seed, gid, e.cycle, RNG_ACTION, 3);
+          av2.x = clampf(-1.0f, av2.x + epsilon * u11(w2.x), 1.0f);
+          av2.y = clampf(-1.0f, av2.y + epsilon * u11(w2.y), 1.0f);
+          av2.z = clampf(-1.0f, av2.z + epsilon * u11(w2.z), 1.0f);
+          av2.w = clampf(-1.0f, av2.w + epsilon * u11(w2.w), 1.0f);
+        }
       }
+      if constexpr (kActDim == 8) {
+        if (T.actions_f && valid) {  // 32-byte rows of a 16-byte aligned buffer (s2d_api.cu checks)
+          float4* dst = reinterpret_cast<float4*>(T.actions_f + (static_cast<int64_t>(k) * n + i) * 8);
+          dst[0] = av;
+          dst[1] = av2;
+        }
+        out.reward_sum = 0.0f;
+        const float4 c = parameterized_command(av, av2);
+        rs = substep<SCN, S2D_ACT_COMMAND, SP, true>(e, P, sp, gid, i, c.x, c.y, c.z, c.w, out);
+      } else {
       if (T.actions_f && valid) {
         float* dst = T.actions_f + (static_cast<int64_t>(k) * n + i) * kActDim;
         dst[0] = av.x;
@@ -304,6 +330,7 @@ __global__ void __launch_bounds__(kBlock, S2D_ROLLOUT_MIN_BLOCKS)
       out.reward_sum = 0.0f;
       rs = substep<SCN, ACT, SP, true>(e, P, sp, gid, i, av.x, kActDim == 4 ? av.y : 0.f, kActDim == 4 ? av.z : 0.f,
                                        kActDim == 4 ? av.w : 0.f, out, kActDim == 1 ? P.sincos_memo : nullptr);
+      }
     } else {
     if (epsilon > 0.0f) {  // exploration: the same counter stream as the mma.sync kernel
       const uint4 w = philox4x32_10(P.seed, gid, e.cycle, RNG_ACTION, 1);
@@ -353,6 +380,12 @@ __global__ void __launch_bounds__(kBlock, S2D_ROLLOUT_MIN_BLOCKS)
   __syncthreads();
   if (warp == 0) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, 128;" ::"r"(s.tmem_base) : "memory");
 }
+
+// SHOOT + S2D_ACT_PARAMETERIZED (s2d_shoot_param.cu): step_kernel and rollout_mlp_tc5_kernel for the constants variant
+// `var` (kVarRuntime, kVarDefault, kVarNoisy); cudaErrorInvalidValue, and no launch, for any other.
+cudaError_t launch_shoot_param(int var, int grid, const KernelParams& kp, int k_substeps, cudaStream_t s);
+cudaError_t launch_shoot_param_actor(int var, int grid, const KernelParams& kp, int k_substeps, const MlpWeights& w,
+                                     float noise, const TrajOut& traj, cudaStream_t s);
 
 #endif  // !S2D_HOST_EMU
 

@@ -397,6 +397,18 @@ __device__ __forceinline__ void reset_episode(Episode& e, const KernelParams& P,
   finish_reset<SCN>(e, P, sp, gid);
 }
 
+// S2D_ACT_PARAMETERIZED (SHOOT; spec: include/soccer2d.h): the row a[0..7], as two float4 halves, -> the
+// S2D_ACT_COMMAND row it stands for.  clampf turns a NaN into +1; the largest weight wins, ties to the lower index.
+__device__ __forceinline__ float4 parameterized_command(float4 lo, float4 hi) {
+  const float wd = clampf(-1.0f, lo.x, 1.0f), wt = clampf(-1.0f, lo.y, 1.0f), wk = clampf(-1.0f, lo.z, 1.0f);
+  if (wd >= wt && wd >= wk)
+    return make_float4(static_cast<float>(S2D_CMD_DASH), (clampf(-1.0f, lo.w, 1.0f) + 1.0f) * 50.0f,
+                       clampf(-1.0f, hi.x, 1.0f) * 180.0f, 0.0f);
+  if (wt >= wk) return make_float4(static_cast<float>(S2D_CMD_TURN), clampf(-1.0f, hi.y, 1.0f) * 180.0f, 0.0f, 0.0f);
+  return make_float4(static_cast<float>(S2D_CMD_KICK), (clampf(-1.0f, hi.z, 1.0f) + 1.0f) * 50.0f,
+                     clampf(-1.0f, hi.w, 1.0f) * 180.0f, 0.0f);
+}
+
 // ONE env-step = what Soccer2DEnv.step does: decode the action, run the server cycle, score it; when the
 // episode ends, record it and (auto_reset) start the next one (placement, idle cycle, priming check).
 //   discrete:   (a0..a3) = the action's table entry {cmd, power, lowered direction, dash rate}
@@ -516,6 +528,9 @@ constexpr int kBlock = S2D_BLOCK;
 #ifndef S2D_MIN_BLOCKS
 #define S2D_MIN_BLOCKS 8  // resident blocks per SM the step kernel is compiled for (register budget)
 #endif
+// S2D_ACT_PARAMETERIZED: with the 64 registers of 8 blocks its runtime-constant and noisy kernels spill; with 7 (72
+// registers) none does
+constexpr int kParamMinBlocks = 7;
 
 // K lockstep cycles of every env in one launch; state stays in registers in between.
 // actions[N][K] (uint8 / float) or [N][K][4] (float): a lane's K actions are contiguous in memory; the first
@@ -603,7 +618,8 @@ __device__ __forceinline__ void end_of_episode(Episode& e, const KernelParams& P
 }
 
 template <int SCN, int ACT, int VAR>
-__global__ void __launch_bounds__(kBlock, S2D_MIN_BLOCKS) step_kernel(const __grid_constant__ KernelParams P, const int K) {
+__global__ void __launch_bounds__(kBlock, ACT == S2D_ACT_PARAMETERIZED ? kParamMinBlocks : S2D_MIN_BLOCKS)
+    step_kernel(const __grid_constant__ KernelParams P, const int K) {
   using SP = typename VariantSP<VAR>::type;
   const SP sp(P.cc);
   __shared__ __align__(16) float s_stage[kBlock / 32][32 * kObsDim];
@@ -622,7 +638,16 @@ __global__ void __launch_bounds__(kBlock, S2D_MIN_BLOCKS) step_kernel(const __gr
   // nothing), so that the warp can handle the end of an episode together, see end_of_episode.
   const int64_t il = valid ? i : n - 1;
   load_episode(P.state, n, il, e);
-  if (ACT == S2D_ACT_DISCRETE) {
+  if constexpr (ACT == S2D_ACT_PARAMETERIZED) {
+    // SHOOT: 32-byte rows, translated to the command row (s2d_shoot_param.cu instantiates these kernels)
+    const float4* act = static_cast<const float4*>(P.actions) + il * K * 2;
+#pragma unroll 1
+    for (int k = 0; k < K; ++k) {
+      const float4 c = parameterized_command(__ldg(act + 2 * k), __ldg(act + 2 * k + 1));
+      const int rs = substep<SCN, S2D_ACT_COMMAND, SP, true>(e, P, sp, gid, i, c.x, c.y, c.z, c.w, out);
+      end_of_episode<SCN>(e, P, sp, gid, i, valid, rs, out);
+    }
+  } else if (ACT == S2D_ACT_DISCRETE) {
     // ReachBall: bodies are whole degrees (placement) and never turn, dash directions are snapped to whole degrees:
     // the dash's sin / cos come from the memo (s2d_math.cuh; 5.8 KB, it stays in L1 next to the action table) when
     // the launch is long enough for that to matter.

@@ -4,7 +4,8 @@ Not part of the reference (whose only scenario is ReachBall); it exists to exerc
 kickable-area test and goal / ball-out detection behind the same gym API.  The scenario contract (reset, reward,
 done, result names) is specified in include/soccer2d.h and implemented in csrc/s2d_scenarios.cuh (check_shoot).
 Observation: the same 10 values as ReachBall.  Actions: Discrete(action_space_size) = dashes + `kick_actions` kicks,
-or proto-style commands with use_command_action=True (Dash / Turn / Kick / Body_GoToPoint).
+proto-style commands with use_command_action=True (Dash / Turn / Kick / Body_GoToPoint), or with
+use_parameterized_action=True HFO's parameterized Box(8): weights of dash / turn / kick and their continuous arguments.
 """
 from __future__ import annotations
 

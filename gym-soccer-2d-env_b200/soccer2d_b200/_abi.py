@@ -8,13 +8,14 @@ from __future__ import annotations
 import ctypes as C
 import os
 
-ABI_VERSION = 13
+ABI_VERSION = 14
 MAX_PIPELINE_SLOTS = 4
 
 # ---- constants (mirror include/soccer2d.h) ----------------------------------------------------------
 S2D_OK, S2D_ERR_INVALID, S2D_ERR_UNBOUND, S2D_ERR_CUDA, S2D_ERR_NO_DEVICE = 0, -1, -2, -3, -4
 SCENARIO_REACHBALL, SCENARIO_SHOOT, SCENARIO_FULLGAME = 0, 1, 2
 ACT_DISCRETE, ACT_CONTINUOUS, ACT_TURNING, ACT_COMMAND = 0, 1, 2, 3
+ACT_PARAMETERIZED = 4  # SHOOT: dash / turn / kick with continuous arguments, 8 floats per row
 CMD_NONE, CMD_DASH, CMD_TURN, CMD_KICK, CMD_GOTO = 0, 1, 2, 3, 4
 CMD_TURN_TO_POINT, CMD_TURN_TO_BALL, CMD_TURN_TO_ANGLE, CMD_KICK_ONE_STEP, CMD_STOP_BALL, CMD_INTERCEPT = 5, 6, 7, 8, 9, 10
 CMD_TACKLE, CMD_CATCH, CMD_SMART_KICK = 11, 12, 13

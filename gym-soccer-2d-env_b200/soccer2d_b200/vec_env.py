@@ -28,10 +28,11 @@ REACHBALL_DEFAULTS = dict(
     ball_direction=0, min_distance_to_ball=5.0, max_steps=200, use_continuous_action=True, action_space_size=16,
     use_turning=False)
 
-# 1v0 shoot-on-goal (BASELINE configs[2]; spec in include/soccer2d.h): Discrete(24) = 16 dashes + 8 kicks by default
+# 1v0 shoot-on-goal (BASELINE configs[2]; spec in include/soccer2d.h): Discrete(24) = 16 dashes + 8 kicks by default;
+# use_parameterized_action=True: Box(-1, 1, (8,)) = HFO's dash / turn / kick with continuous arguments
 SHOOT_DEFAULTS = dict(
     change_ball_position=True, change_ball_velocity=False, ball_position_x=0, ball_position_y=0, ball_speed=0,
-    ball_direction=0, max_steps=200, action_space_size=24, kick_actions=8)
+    ball_direction=0, max_steps=200, action_space_size=24, kick_actions=8, use_parameterized_action=False)
 
 # full match, up to 11 v 11 (BASELINE configs[3]; spec in include/soccer2d.h): command actions for every player
 FULLGAME_DEFAULTS = dict(players_per_side=11, half_time_cycles=3000)
@@ -231,6 +232,8 @@ class Soccer2DVecEnv(_VecEnvBase):
             self.num_players = 2 * cfg.players_per_side
         if use_command_action:
             cfg.action_mode = _abi.ACT_COMMAND
+        elif self.kw.get("use_parameterized_action", False):
+            cfg.action_mode = _abi.ACT_PARAMETERIZED
         elif self.kw.get("use_continuous_action", False):
             cfg.action_mode = _abi.ACT_TURNING if self.kw["use_turning"] else _abi.ACT_CONTINUOUS
         else:
@@ -269,6 +272,8 @@ class Soccer2DVecEnv(_VecEnvBase):
         elif cfg.action_mode == _abi.ACT_TURNING:
             self.action_space = Box(low=np.array([-1, -1, -1, -1], dtype=np.float32),
                                     high=np.array([1, 1, 1, 1], dtype=np.float32), dtype=np.float32)
+        elif cfg.action_mode == _abi.ACT_PARAMETERIZED:  # [w_dash, w_turn, w_kick, dash power, dash dir, turn dir, kick power, kick dir]
+            self.action_space = Box(low=-1, high=1, shape=(8,), dtype=np.float32)
         elif cfg.action_mode == _abi.ACT_CONTINUOUS:
             self.action_space = Box(low=-1, high=1, shape=(1,), dtype=np.float32)
         else:
@@ -294,6 +299,8 @@ class Soccer2DVecEnv(_VecEnvBase):
             self.actions = io((n, k), torch.float32)
         elif self.scenario == "fullgame":
             self.actions = io((n, k, self.num_players, 4), torch.float32)
+        elif cfg.action_mode == _abi.ACT_PARAMETERIZED:
+            self.actions = io((n, k, 8), torch.float32)
         else:
             self.actions = io((n, k, 4), torch.float32)
         assert self.actions.numel() * self.actions.element_size() == self.lib.s2d_action_bytes(C.byref(cfg)) * k
@@ -730,14 +737,15 @@ class Soccer2DVecEnv(_VecEnvBase):
     def rollout_actor(self, layers, k: int | None = None, noise: float = 0.0, traj: dict | None = None,
                       precision: str = "tf32") -> None:
         """`k` cycles of observe -> actor(obs) -> Box action -> step in ONE launch (ReachBall with the Box(1) or the Box(4)
-        turning action space): the DDPG counterpart of `rollout_mlp` (s2d_rollout_actor_collect).  `layers` = [(weight,
-        bias)] * 3 of a 64-64 ReLU MLP whose last layer has action_dim rows; tanh is applied in the kernel.  `noise`: the
-        half-width of a uniform exploration noise.  `traj`: time-major tensors, any of obs float32 [k + 1, N, 10],
-        actions float32 [k, N, action_dim], reward float32 [k, N], done uint8 [k, N].  `precision`: "tf32" (default:
-        tcgen05.mma, accumulators in tensor memory) or "tf32_mma_sync" (the warp-level kernel of round 1)."""
+        turning action space, Shoot with the Box(8) parameterized one): the DDPG counterpart of `rollout_mlp`
+        (s2d_rollout_actor_collect).  `layers` = [(weight, bias)] * 3 of a 64-64 ReLU MLP whose last layer has
+        action_dim rows; tanh is applied in the kernel.  `noise`: the half-width of a uniform exploration noise on every
+        component.  `traj`: time-major tensors, any of obs float32 [k + 1, N, 10], actions float32 [k, N, action_dim],
+        reward float32 [k, N], done uint8 [k, N].  `precision`: "tf32" (default: tcgen05.mma, accumulators in tensor
+        memory) or "tf32_mma_sync" (the warp-level kernel of round 1; not for Shoot's parameterized actions)."""
         k = self.substeps if k is None else int(k)
         self._user_dirty = True
-        ad = 4 if self.action_mode == _abi.ACT_TURNING else 1
+        ad = {_abi.ACT_TURNING: 4, _abi.ACT_PARAMETERIZED: 8}.get(self.action_mode, 1)
         ptrs = []
         for (w, b), shape in zip(layers, ((64, self.obs_dim), (64, 64), (ad, 64))):
             if tuple(w.shape) != shape or tuple(b.shape) != shape[:1]:

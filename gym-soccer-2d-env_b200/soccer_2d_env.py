@@ -226,10 +226,10 @@ class Soccer2DEnv(Env):
                 raise ValueError(f"discrete action {a} outside Discrete({n})")
             return np.array([[a]], dtype=np.uint8)
         a = np.asarray(action, dtype=np.float32).reshape(-1)
-        want = 4 if mode in (_abi.ACT_TURNING, _abi.ACT_COMMAND) else 1
+        want = 8 if mode == _abi.ACT_PARAMETERIZED else 4 if mode in (_abi.ACT_TURNING, _abi.ACT_COMMAND) else 1
         if a.size != want:
             raise ValueError(f"expected an action with {want} value(s), got shape {np.asarray(action).shape}")
-        return a.reshape((1, 1, 4) if want == 4 else (1, 1))
+        return a.reshape((1, 1, want) if want > 1 else (1, 1))
 
     @property
     def distance_to_ball(self) -> float:

@@ -42,7 +42,7 @@
 extern "C" {
 #endif
 
-#define S2D_ABI_VERSION 13
+#define S2D_ABI_VERSION 14
 
 /* error codes */
 #define S2D_OK 0
@@ -167,6 +167,17 @@ extern "C" {
 #define S2D_ACT_CONTINUOUS 1 /* float  [N][K][1]   Box(-1,1,(1,)): Dash(100, a*180)               (REACHBALL)   */
 #define S2D_ACT_TURNING 2    /* float  [N][K][4]   [turn_prob, turn_angle, dash_prob, dash_angle] (REACHBALL)   */
 #define S2D_ACT_COMMAND 3    /* float4 [N][K][P]   {cmd, a, b, c} per player: see S2D_CMD_* (proto PlayerAction) */
+#define S2D_ACT_PARAMETERIZED 4 /* float [N][K][8] dash / turn / kick with continuous arguments (SHOOT; spec below)  */
+
+/* SHOOT + S2D_ACT_PARAMETERIZED (the HFO parameterized action space without tackle; not in the reference - this is the spec).
+ * Row a[0..7]; every component is first clamped: c(x) = max(-1, min(x, 1)) (fminf / fmaxf order: a NaN becomes +1).
+ *   a[0], a[1], a[2]  weights of dash, turn, kick: the largest c() selects the command, ties to the lower index.
+ *   The row then IS the S2D_ACT_COMMAND row (fp32, one rounding per operation as written):
+ *     dash  {DASH, (c(a[3]) + 1) * 50, c(a[4]) * 180, 0}   power 0..100, direction lowered by dash_direction as every dash
+ *     turn  {TURN, c(a[5]) * 180, 0, 0}
+ *     kick  {KICK, (c(a[6]) + 1) * 50, c(a[7]) * 180, 0}   no effect unless the ball is kickable, as every kick
+ *   No randomness: unlike S2D_ACT_TURNING's sampled choice, the same row in the same state gives the same command.
+ *   Reset, reward, done, results and the 10-float observation are SHOOT's, unchanged.  32 bytes per env and cycle. */
 
 /* S2D_ACT_COMMAND: cmd stored as a float; arguments as in the proto messages */
 #define S2D_CMD_NONE 0 /* no body command this cycle                                  */
@@ -495,7 +506,8 @@ int s2d_rollout_mlp_collect(S2DHandle h, const S2DMlpPolicy* policy, int k_subst
                             const S2DTrajectory* trajectory, void* stream);
 
 /* The same for a deterministic actor (DDPG, ddpg_stable_baselines3.py / dqn_ddpg_stable_baselines3.py): REACHBALL with
- * S2D_ACT_CONTINUOUS (Box(1)) or S2D_ACT_TURNING (Box(4)).  `actor` = obs -> 64 -> 64 -> action_dim with ReLU and a
+ * S2D_ACT_CONTINUOUS (Box(1)) or S2D_ACT_TURNING (Box(4)), or SHOOT with S2D_ACT_PARAMETERIZED (Box(8); precision 0
+ * only, and `actions_f` 16-byte aligned).  `actor` = obs -> 64 -> 64 -> action_dim with ReLU and a
  * final tanh (w3: [action_dim][64]); `noise` = half-width of a uniform exploration noise added to every component
  * before the clip to [-1, 1] (0: the deterministic policy).  `trajectory` may be NULL; its `actions` is not used. */
 int s2d_rollout_actor_collect(S2DHandle h, const S2DMlpPolicy* actor, int k_substeps, float noise,
