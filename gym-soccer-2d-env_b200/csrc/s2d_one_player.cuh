@@ -474,9 +474,9 @@ __device__ __noinline__ inline float4 resolve_ball_player_overlap_backtrace(floa
 }
 
 template <class SP>
-// (dx, dy) = ball - player and d2 = dx*dx + dy*dy come from the caller, which re-uses them for the reward when
-// nothing collided (the common case).  Returns true when something was moved.
-__device__ __forceinline__ bool collide_ball_player(Episode& e, float d2, const SP& sp) {
+// (dx, dy) = ball - player and d2 = dx*dx + dy*dy come from the caller, which re-uses them for the reward.  A collision
+// (rare) moves the objects and recomputes the three in its own branch, so that the common cycle does not pay for it.
+__device__ __forceinline__ void collide_ball_player(Episode& e, float& dx, float& dy, float& d2, const SP& sp) {
   uint32_t hit = 0;
   if (d2 < sp.collide_r2()) {
     hit = S2D_FLAG_BALL_COLLIDED | S2D_FLAG_PLAYER_COLLIDED;
@@ -495,9 +495,11 @@ __device__ __forceinline__ bool collide_ball_player(Episode& e, float d2, const 
     e.bvy *= -0.1f;
     e.vx *= -0.1f;
     e.vy *= -0.1f;
+    dx = e.bx - e.px;
+    dy = e.by - e.py;
+    d2 = dx * dx + dy * dy;
   }
   e.flags = (e.flags & ~(S2D_FLAG_BALL_COLLIDED | S2D_FLAG_PLAYER_COLLIDED)) | hit;
-  return hit != 0;
 }
 
 // Player::updateStamina, written with selects instead of nested branches.
@@ -555,11 +557,7 @@ __device__ __forceinline__ void simulate_cycle(Episode& e, int cmd, float power,
   dx = e.bx - e.px;
   dy = e.by - e.py;
   d2 = dx * dx + dy * dy;
-  if (collide_ball_player(e, d2, sp)) {
-    dx = e.bx - e.px;
-    dy = e.by - e.py;
-    d2 = dx * dx + dy * dy;
-  }
+  collide_ball_player(e, dx, dy, d2, sp);
   update_stamina(e, sp);
   e.cycle += 1u;
 }

@@ -326,10 +326,15 @@ __device__ __forceinline__ Placement draw_placement_warp(const KernelParams& P, 
       const uint32_t qx = __shfl_sync(full, w.x, src), qy = __shfl_sync(full, w.y, src), qz = __shfl_sync(full, w.z, src),
                      qw = __shfl_sync(full, w.w, src);
       const float s_try = u32_to_unit((t & 1) ? qz : qx) * 3.0f;
-      const float d_try = static_cast<float>(u32_to_int((t & 1) ? qw : qy, 0, 360));
+      const int deg = u32_to_int((t & 1) ? qw : qy, 0, 360);
       float tsn, tcs;
-      if (MEMO && P.sincos_memo) sincos_deg_memo(d_try, P.sincos_memo, tsn, tcs);  // whole degrees in [0, 360]: always a hit
-      else sincos_deg(d_try, tsn, tcs);
+      if (MEMO && P.sincos_memo) {  // whole degrees in [0, 360]: the memo entry sincos_deg_memo would hit, indexed directly
+        const float2 m = __ldg(P.sincos_memo + (deg + kSinCosMemoHalf));
+        tsn = m.x;
+        tcs = m.y;
+      } else {
+        sincos_deg(static_cast<float>(deg), tsn, tcs);
+      }
       const unsigned ok = __ballot_sync(full, have && ball_stays_inside(P, pl.bx, pl.by, s_try, tsn, tcs));
       if (ok) {
         const int first = __ffs(ok) - 1;
@@ -424,6 +429,7 @@ __device__ __forceinline__ int substep(Episode& e, const KernelParams& P, const 
   constexpr bool kTurns = ACT == S2D_ACT_TURNING || ACT == S2D_ACT_COMMAND;
   constexpr bool kKicks = ACT == S2D_ACT_COMMAND || SCN == S2D_SCENARIO_SHOOT;
   e.step_number += 1;  // reach_ball_env.py:55
+  opaque(e.step_number);  // the time-out test reads the new count (not old >= max_steps, which keeps the old one alive)
   int cmd = S2D_CMD_DASH;
   float power = 100.0f, dir, rate;
   if (ACT == S2D_ACT_DISCRETE) {
@@ -572,6 +578,9 @@ __device__ __forceinline__ void end_of_episode(Episode& e, const KernelParams& P
   const bool done = rs != S2D_RESULT_NONE;
   unsigned pending = __ballot_sync(full, done);
   if (pending == 0u) return;
+  // the ending reads the cycle's clock and flags, not values re-derived from those before the cycle (s2d_math.cuh)
+  opaque(e.cycle);
+  opaque(e.flags);
   if (done) {
     if (e.flags & S2D_FLAG_DONE) {
       out.report_only(rs);
@@ -592,10 +601,8 @@ __device__ __forceinline__ void end_of_episode(Episode& e, const KernelParams& P
     // the usual case, ONE lane due: it places its new episode and runs the idle cycle in one piece, so that the
     // compiler sees a player at rest with full stamina there (most of that cycle folds away)
     const int lane = threadIdx.x & 31, src = __ffs(pending) - 1;
-    const uint32_t g_lo = __shfl_sync(full, static_cast<uint32_t>(gid), src);
-    const uint32_t g_hi = __shfl_sync(full, static_cast<uint32_t>(gid >> 32), src);
     const uint32_t episode = __shfl_sync(full, e.episode, src);
-    const Placement pl = draw_placement_warp<MEMO>(P, (static_cast<uint64_t>(g_hi) << 32) | g_lo, episode, lane);
+    const Placement pl = draw_placement_warp<MEMO>(P, gid - lane + src, episode, lane);  // the lanes' gids are consecutive
     if (done) {
       apply_placement(e, pl, sp);
       finish_reset<SCN>(e, P, sp, gid);
@@ -605,10 +612,8 @@ __device__ __forceinline__ void end_of_episode(Episode& e, const KernelParams& P
     do {
       const int src = __ffs(pending) - 1;
       pending &= pending - 1u;
-      const uint32_t g_lo = __shfl_sync(full, static_cast<uint32_t>(gid), src);
-      const uint32_t g_hi = __shfl_sync(full, static_cast<uint32_t>(gid >> 32), src);
       const uint32_t episode = __shfl_sync(full, e.episode, src);
-      const Placement pl = draw_placement_warp<MEMO>(P, (static_cast<uint64_t>(g_hi) << 32) | g_lo, episode, lane);
+      const Placement pl = draw_placement_warp<MEMO>(P, gid - lane + src, episode, lane);
       if (lane == src) apply_placement(e, pl, sp);
     } while (pending);
     if (done) finish_reset<SCN>(e, P, sp, gid);

@@ -5,12 +5,15 @@
 
 Walks from address START to address STOP (hex, both counted): unconditional branches are followed, a conditional one
 (`@P BRA`, `BRA P`, `BRA.U`) only when its address is listed in TAKEN, calls are counted as one instruction and not
-entered (the cold paths are out-of-line functions)."""
+entered (the cold paths are out-of-line functions).  ADDR:N in TAKEN takes that branch its first N times only (a loop
+that runs N + 1 times, such as the draw loop of a two-lane ending)."""
 import re
 import sys
 
 
 def walk(path, start, stop, taken):
+    """taken: {address: times the branch is taken (None: always)}"""
+    taken = dict(taken)
     ins = {}
     for line in open(path):
         m = re.match(r"\s*/\*([0-9a-f]{4,})\*/\s+(.*?)\s*;", line)
@@ -25,7 +28,9 @@ def walk(path, start, stop, taken):
         m = re.search(r"\bBRA(?:\.U)?\s+(?:!?U?P\d, )?0x([0-9a-f]+)", text)
         if m:
             conditional = text.startswith("@") or "BRA.U" in text or re.search(r"BRA\s+!?P\d,", text)
-            if not conditional or pc in taken:
+            if not conditional or (pc in taken and taken[pc] != 0):
+                if conditional and taken[pc] is not None:
+                    taken[pc] -= 1
                 pc = int(m.group(1), 16)
                 continue
         pc += 16
@@ -33,5 +38,8 @@ def walk(path, start, stop, taken):
 
 
 if __name__ == "__main__":
-    taken = {int(a, 16) for a in sys.argv[4].split(",")} if len(sys.argv) > 4 and sys.argv[4] else set()
+    taken = {}
+    for a in (sys.argv[4].split(",") if len(sys.argv) > 4 and sys.argv[4] else []):
+        addr, _, times = a.partition(":")
+        taken[int(addr, 16)] = int(times) if times else None
     print(walk(sys.argv[1], int(sys.argv[2], 16), int(sys.argv[3], 16), taken))
